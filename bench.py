@@ -2,6 +2,7 @@
 """Headline benchmark: episodes/sec, 5-way 5-shot 15-query, waveform -> logits.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mode eval|train|eval10k]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json `metric`; SURVEY.md 8d, config C1 = config/proto_5shot_iid.yaml): ProtoNet on
 Conv64F, 5w5s15q = 100 clips per episode, each clip 5 s @ 16 kHz (L = 80 000) -> log-mel [1,128,157]
@@ -41,6 +42,17 @@ Collective-bearing modes (their own JSON line, same contract keys):
                   reference's 1-float accuracy all-reduce per step stays (utils.py:116-118).
   --mode eval10k  BASELINE configs[1]: ProtoNet/ResNet-12 5w1s15q, 10 000 episodes sharded over the ranks, ONE
                   all_gather of the per-episode accuracies + the 95 % CI at the end (test.py:210) inside the timing.
+
+`--steps` is the number of timed steps of eval, train and --impl reference.  eval10k times the whole job instead,
+--episodes / (episodes per step * ranks) steps, and refuses --steps.
+
+`--dump-outputs DIR` writes what the timed path returned, on rank 0, as DIR/<name>.npy (float32, float64 where the
+path computes in float64): for the last timed step, eval and --impl reference `logits` and `accuracy_pct`, train
+`logits`, `loss` and `accuracy_pct`; for the whole eval10k job, `episode_accuracy_pct` (every episode, in global
+order) and `accuracy_mean_ci95`.  Inputs and weights are seeded, so the same arguments give the same inputs on every
+run and two builds can be compared output for output.  With equal --steps and episodes per step, the eval and
+--impl reference dumps come from the same waveforms, unless --ref-seconds made the reference arm run fewer episodes
+per step (its JSON note then says "bounded below").
 """
 import argparse
 import json
@@ -75,7 +87,7 @@ CONV3_FLOP_PER_CLIP = 2 * 9 * 64 * 64 * (42 * 52 + 14 * 17)  # blocks 2 + 3: 3x3
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 100; not in eval10k)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--mode", default="eval", choices=["eval", "train", "eval10k"])
@@ -91,7 +103,25 @@ def parse():
     ap.add_argument("--ref-seconds", type=float, default=240.0,
                     help="--impl reference: bound of the whole run (the driver's --steps 20 --warmup 5 at the B200 arm's "
                          "32 episodes per step needs about 150 s on the box's 16 host threads)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned as DIR/<name>.npy (see the module docstring)")
+    args = ap.parse_args()
+    if args.mode == "eval10k" and args.impl == "b200":
+        if args.steps is not None:
+            ap.error("--mode eval10k runs --episodes / (episodes per step * ranks) steps; set --episodes, not --steps")
+    elif args.steps is None:
+        args.steps = 100
+    elif args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(directory, arrays):
+    """Write {name: tensor or array} as directory/<name>.npy, float64 kept, every other dtype as float32."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a.detach().cpu() if hasattr(a, "detach") else a)
+        np.save(os.path.join(directory, name + ".npy"), a if a.dtype == np.float64 else a.astype(np.float32))
 
 
 def mean_std():
@@ -215,8 +245,10 @@ def run_reference(args, rank):
         path.episodes(wav[i % 2], e_ref)
     t0 = time.perf_counter()
     for i in range(args.steps):
-        path.episodes(wav[i % 2], e_ref)
+        output, acc = path.episodes(wav[i % 2], e_ref)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": output, "accuracy_pct": acc})
     value = args.steps * e_ref / dt
     cfg = base_config(e_ref, e_ref * CLIPS_PER_EPISODE, 1)
     cfg["note"] = ("CPU oracle port of the reference path; runs on rank 0's host cores only, whatever --gpus says; "
@@ -502,6 +534,8 @@ def run_eval(args, rank, world, local_rank):
         launches = ops.launch_count() - launches0
         logmel_ms = ranks.max(float(np.mean([a.elapsed_time(b) for a, b in lm_events])))
         acc_dev = float(acc.item())
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"logits": output, "accuracy_pct": acc})
 
         # ---- end to end through the public call: `e2e`
         run_e2e(args.warmup, host)
@@ -724,13 +758,15 @@ def run_train(args, rank, world, local_rank):
         loss.backward()
         afs_dist.all_reduce_gradients(model.parameters())           # ONE flat collective (trainer.py:504-509)
         opt.step()
-        return acc, loss
+        return output, acc, loss
 
     for i in range(args.warmup):
         step(i)
     l0 = ops.launch_count()
-    ms, (acc, loss) = timed(ranks, step, args.steps)
+    ms, (output, acc, loss) = timed(ranks, step, args.steps)
     launches = ops.launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"logits": output, "loss": loss, "accuracy_pct": acc})
     # replicas must stay identical: the same parameters on every rank after K data-parallel steps
     checksum = torch.stack([p.detach().double().sum() for p in model.parameters()]).sum()
     spread = 0.0
@@ -823,6 +859,8 @@ def run_eval10k(args, rank, world, local_rank):
         launches = ops.launch_count() - l0
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"episode_accuracy_pct": acc_all, "accuracy_mean_ci95": np.array([m, h])})
     emit({"metric": "episodes/sec (5w1s15q ResNet-12, waveform->logits, %d episodes incl. accuracy gather + 95%% CI)" % n_total,
           "value": n_total / (ms * 1e-3), "unit": "episodes/sec", "n_gpus": world, "steps": steps, "warmup": args.warmup,
           "ms_per_step": ms / steps, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,

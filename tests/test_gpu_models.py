@@ -921,3 +921,28 @@ def test_pool3_linear_matches_pool_and_addmm(cuda, N, H, W, J):
     assert not ops.pool3_linear_supported(torch.empty(1, 64, 6, 5), 1600)  # pooled map larger than one pixel
     with pytest.raises(ValueError):
         ops.pool3_linear(torch.zeros(2, 32, 4, 5, device=cuda), w, b)
+
+
+def test_bench_dump_outputs_match_the_cpu_reference_arm(cuda, tmp_path):
+    """`bench.py --dump-outputs`: the logits and accuracy of the B200 arm's last timed step (default precision) agree
+    with those of the CPU oracle arm, which reads the same seeded waveforms at equal --steps and episodes per step."""
+    import os
+    import subprocess
+    import sys
+
+    from conftest import ROOT
+
+    def run(impl):
+        out = tmp_path / impl
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", impl, "--steps", "2",
+                            "--warmup", "1", "--episodes-per-step", "1", "--no-extras", "--no-cpu-baseline",
+                            "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        return np.load(out / "logits.npy"), np.load(out / "accuracy_pct.npy")
+
+    got, acc = run("b200")
+    want, want_acc = run("reference")
+    assert got.dtype == np.float32 and got.shape == want.shape == (5 * 15, 5)
+    assert np.abs(got - want).max() < 2e-2 * np.abs(want).max()  # TF32 backbone against the fp32 oracle, as smoke()
+    assert (got.argmax(1) == want.argmax(1)).mean() >= 0.97
+    assert abs(float(acc) - float(want_acc)) <= 100.0 * 2 / 75

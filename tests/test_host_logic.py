@@ -62,7 +62,7 @@ def test_model_contract_on_cpu():
 
 def test_finetuning_model_contract():
     """FinetuningModel (finetuning_model.py:10-31): model_type, the three abstract methods, sub_optimizer from a
-    {"name", "kwargs"} block -- checked against the reference class when it is importable."""
+    {"name", "kwargs"} block."""
     from audio_fewshot_b200 import model as arch
 
     class Probe(arch.FinetuningModel):
@@ -84,13 +84,15 @@ def test_finetuning_model_contract():
     opt = m.sub_optimizer(m.classifier, {"name": "SGD", "kwargs": {"lr": 0.01, "momentum": 0.9}})
     assert isinstance(opt, torch.optim.SGD) and opt.param_groups[0]["momentum"] == 0.9
     assert isinstance(m.sub_optimizer(m.classifier, {"name": "Adam", "kwargs": None}), torch.optim.Adam)
-    from oracle import ref_import
-    if ref_import.reference_available():
-        ref = ref_import.import_reference()
-        import importlib
-        ref_cls = importlib.import_module("libfewshot_core.model.finetuning.finetuning_model").FinetuningModel
-        want = {n for n in vars(ref_cls) if not n.startswith("_")}
-        assert want <= {n for n in dir(arch.FinetuningModel)}, want
+
+
+def test_finetuning_model_has_the_live_reference_public_names(reference):
+    import importlib
+
+    from audio_fewshot_b200 import model as arch
+    ref_cls = importlib.import_module("libfewshot_core.model.finetuning.finetuning_model").FinetuningModel
+    want = {n for n in vars(ref_cls) if not n.startswith("_")}
+    assert want <= {n for n in dir(arch.FinetuningModel)}, want
 
 
 def test_sharding_is_a_partition():
@@ -180,13 +182,14 @@ def test_tta_helpers_match_live_reference(reference):
         assert torch.equal(a, b)
 
 
-def test_bench_reference_arm_line_and_no_cuda_refusal():
+def test_bench_reference_arm_line_and_no_cuda_refusal(tmp_path):
     """`bench.py --impl reference` (the oracle port timed on the host cores) prints ONE JSON line with the contract's
-    keys; the B200 arm refuses to run without a CUDA device instead of falling back."""
+    keys and dumps its last step's outputs; the B200 arm refuses to run without a CUDA device instead of falling back."""
     import json
     env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
-                          "--warmup", "0", "--episodes-per-step", "2"], capture_output=True, text=True, env=env, timeout=300)
+                          "--warmup", "0", "--episodes-per-step", "2", "--dump-outputs", str(tmp_path / "dump")],
+                         capture_output=True, text=True, env=env, timeout=300)
     assert out.returncode == 0, out.stderr[-500:]
     lines = [l for l in out.stdout.splitlines() if l.strip()]
     assert len(lines) == 1
@@ -198,6 +201,9 @@ def test_bench_reference_arm_line_and_no_cuda_refusal():
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert "workload" in d["config"] and "model" not in d["config"]
     assert d["config"]["episodes_per_step_per_gpu"] == 2  # the CPU arm runs the B200 arm's step, not one episode
+    logits, acc = np.load(tmp_path / "dump" / "logits.npy"), np.load(tmp_path / "dump" / "accuracy_pct.npy")
+    assert logits.dtype == acc.dtype == np.float32 and logits.shape == (2 * 5 * 15, 5) and acc.shape == ()
+    assert np.isfinite(logits).all() and 0.0 <= acc <= 100.0
     # under torchrun only rank 0 runs the reference arm; the other ranks exit 0 without work or output
     other = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2",
                             "--steps", "1", "--warmup", "0"], capture_output=True, text=True, timeout=300,
