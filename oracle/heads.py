@@ -119,12 +119,13 @@ def dn4_layer(query_feat, support_feat, way_num, shot_num, n_k, return_topk=Fals
 
 def bdcovpool(x, t):
     """reference: BDCovpool, libfewshot_core/model/backbone/utils/bdc_pool.py:69-84.
-    x [B, dim, h, w], t: log-temperature tensor [1,1]."""
+    x [B, dim, h, w], t: log-temperature tensor [1,1].  Runs on x's device and dtype (tests/test_gpu_bdc.py
+    evaluates it in float64 on the GPU at batch sizes the CPU would take seconds over)."""
     B, dim, h, w = x.shape
     M = h * w
     x = x.reshape(B, dim, M)
-    I = torch.eye(dim, dim).view(1, dim, dim).repeat(B, 1, 1).type(x.dtype)  # :74
-    I_M = torch.ones(B, dim, dim).type(x.dtype)  # :75
+    I = torch.eye(dim, dim, device=x.device).view(1, dim, dim).repeat(B, 1, 1).type(x.dtype)  # :74
+    I_M = torch.ones(B, dim, dim, device=x.device).type(x.dtype)  # :75
     x_pow2 = x.bmm(x.transpose(1, 2))  # :76
     dcov = I_M.bmm(x_pow2 * I) + (x_pow2 * I).bmm(I_M) - 2 * x_pow2  # :77
     dcov = torch.clamp(dcov, min=0.0)  # :79
@@ -139,7 +140,7 @@ def triuvec(x):
     The reference's trailing .squeeze() (which drops the batch dim when B == 1) is NOT applied."""
     B, dim, _ = x.shape
     r = x.reshape(B, dim * dim)
-    index = torch.ones(dim, dim).triu().reshape(dim * dim).nonzero(as_tuple=False)
+    index = torch.ones(dim, dim, device=x.device).triu().reshape(dim * dim).nonzero(as_tuple=False)
     return r[:, index].squeeze(-1)
 
 
