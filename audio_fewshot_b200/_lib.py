@@ -78,7 +78,6 @@ SIGNATURES = {
     "afs_conv1_train_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_void_p]),
     "afs_conv3x3_c64_packed_floats": (C.c_size_t, []),
-    "afs_conv3x3_c64_set_pair_mode": (C.c_int, [C.c_int32]),
     "afs_conv3x3_c64_pack_weights": (C.c_int, [C.c_void_p, C.c_void_p]),
     "afs_conv3x3_c64_bn_act_fwd_tf32": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
                                                   C.c_float, C.c_int32, C.c_void_p, C.c_void_p]),

@@ -27,7 +27,7 @@ NVCC_FLAGS = [
     "-Xcompiler", "-fPIC",
     "-Xptxas", "-v",
     "-I", INCLUDE, "-I", CSRC,
-] + (["-DAFS_TC_PROFILE"] if os.environ.get("AFS_TC_PROFILE") == "1" else [])  # development: logmel_tc.cu role timers
+]
 
 
 def _nvcc():

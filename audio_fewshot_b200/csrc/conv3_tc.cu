@@ -33,12 +33,7 @@
 //   warps 12-15 (bf16 kernel) a second epilogue group with its own staging tile: passes 4-7 while the first runs 0-3.
 // All 64x64x9 folded weights stay resident in shared memory (144 KB, pre-packed and TF32-rounded on the host; 72 KB
 // as bf16).  The bf16 instantiation (kind::f16, K = 16: half the MMAs) is the separately stated reduced-precision path.
-// A second kernel below runs the same scheme on CTA pairs (tcgen05 cta_group::2); see its comment for the outcome.
-#include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
-
-#include <atomic>
 
 #include <cuda_bf16.h>
 
@@ -108,7 +103,7 @@ struct Conv3Geom {
   float slope;
 };
 
-// ---- pieces shared by the one-CTA and the CTA-pair kernel --------------------------------------------------------
+// ---- producer and epilogue building blocks of the kernel below -----------------------------------------------------
 
 // One tile's copy plan of a producer thread: thread pair (2j, 2j+1) copies the two 16-byte halves of one pixel's
 // 8-channel group, so a warp reads 16 whole 32-byte sectors and writes 512 contiguous shared-memory bytes per
@@ -394,193 +389,6 @@ conv3x3_c64_tc_kernel(const void* __restrict__ x, const void* __restrict__ wpk, 
   if (warp == 8) tmem_dealloc(tmem_base, kTmemCols);
 }
 
-// ---- CTA pair (cta_group::2) ---------------------------------------------------------------------------------------
-// Two CTAs of a cluster (the two SMs of a TPC) run one M = 256 MMA per step: each supplies the 128 activation rows
-// of ITS tile and only HALF of the weights (32 of the 64 output channels); the tensor cores exchange the halves.
-// Per MMA a CTA now reads 4 KB of A + 1 KB of B from shared memory instead of 4 + 2 KB -- the operand-read pipe is
-// what bounds this kernel -- and the resident weights shrink to 72 KB, which pays for an 8-stage ring.
-// The leader (cluster rank 0) issues every MMA; its "stage full" barriers collect the local producers plus one
-// remote arrival relayed from the peer's producers, its "accumulator empty" barriers the epilogue warps of both
-// CTAs; tcgen05.commit multicasts "stage empty" / "accumulator full" to both CTAs.
-constexpr int kRingP = 8;
-constexpr int kAheadP = 4;
-constexpr uint32_t kTapKcBytesP = 2u * (kC3 / 2) * 16u;   // one (tap, 8-channel group) of one CTA's half: 1 KB
-constexpr uint32_t kWBytesP = 9u * 8u * kTapKcBytesP;      // 73 728 B per CTA
-
-struct BarsP {
-  uint64_t full[kRingP], empty[kRingP];
-  uint64_t acc_full[2], acc_empty[2];
-};
-
-template <int NM>
-__global__ void __launch_bounds__(kThreads3, 1)
-conv3x3_c64_tc_pair_kernel(const float* __restrict__ x, const float* __restrict__ wpk_pair,
-                           const float* __restrict__ shift, float* __restrict__ out, const Conv3Geom g) {
-  extern __shared__ __align__(16) uint8_t s_dyn_raw[];  // [weight half][ring][staging][shift] after 256-byte alignment
-  __shared__ __align__(8) BarsP bars;
-  __shared__ uint32_t s_tmem;
-
-  const int tid = threadIdx.x;
-  const int warp = tid >> 5;
-  const int lane = tid & 31;
-  const uint32_t rank = cluster_ctarank();
-  const bool leader = rank == 0;
-  const uint32_t stage_bytes = static_cast<uint32_t>(g.halo) * 32u;
-  uint8_t* s_dyn = s_dyn_raw + ((256u - (smem_u32(s_dyn_raw) & 255u)) & 255u);
-  const uint32_t w_base = smem_u32(s_dyn);
-  const uint32_t ring_base = w_base + kWBytesP;
-  float* s_stage = reinterpret_cast<float*>(s_dyn + kWBytesP + kRingP * stage_bytes);
-  float* s_shift = s_stage + g.stage_pos * kStagePitch;
-  constexpr uint32_t kTmemCols = NM == 1 ? 128u : (NM == 2 ? 256u : 512u);
-  constexpr uint32_t kIdesc = idesc_tf32(256, kC3);
-
-  {  // this CTA's half of the weights: output channels [32 rank, 32 rank + 32)
-    const uint4* src = reinterpret_cast<const uint4*>(wpk_pair) + static_cast<size_t>(rank) * (kWBytesP / 16);
-    uint4* dst = reinterpret_cast<uint4*>(s_dyn);
-    for (int i = tid; i < static_cast<int>(kWBytesP / 16); i += kThreads3) dst[i] = __ldg(src + i);
-    if (tid < kC3) s_shift[tid] = shift[tid];
-  }
-  if (tid == 0) {
-    for (int s = 0; s < kRingP; ++s) {
-      mbar_init(smem_u32(&bars.full[s]), leader ? 129 : 128);  // local producers (+ the peer's relay on the leader)
-      mbar_init(smem_u32(&bars.empty[s]), NM);                 // multicast commits of the NM issuing warps
-    }
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(smem_u32(&bars.acc_full[s]), NM);
-      mbar_init(smem_u32(&bars.acc_empty[s]), 8);              // epilogue warps of both CTAs (used on the leader)
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 8) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&s_tmem)), "r"(kTmemCols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::);
-  }
-  fence_async_smem();
-  fence_before();
-  __syncthreads();
-  cluster_sync_all();  // both CTAs' barriers, weights and TMEM exist before anyone signals across the pair
-  fence_after();
-  const uint32_t tmem_base = s_tmem;
-  const int total_tiles = g.N * g.tiles_per_img;
-  const int pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;
-  // step j of the pair covers tiles 2*(pair + j*npairs) + {0, 1}; an odd tail tile is paired with a recomputation
-  // of itself whose stores are suppressed
-  auto pair_base = [&](int j) { return 2 * (static_cast<int64_t>(pair) + static_cast<int64_t>(j) * npairs); };
-  auto next_tile = [&](int j) {
-    const int64_t b = pair_base(j);
-    if (b >= total_tiles) return -1;
-    const int64_t t = b + rank;
-    return static_cast<int>(t < total_tiles ? t : total_tiles - 1);
-  };
-
-  if (warp >= 4 && warp < 8) {
-    // ======================= producers (both CTAs fill their own ring) =======================
-    producer_loop<kRingP, kAheadP, 8>(reinterpret_cast<const char*>(x), 4, g, tid - 128, lane, ring_base, stage_bytes,
-                                      bars.full, bars.empty, next_tile);
-  } else if (warp >= 8) {
-    const int m = warp - 8;
-    if (leader) {
-      // ======================= MMA issuers (leader only) =======================
-      if (m < NM && lane == 0) {
-        uint32_t gs = 0, lt = 0;
-        const uint64_t a_desc0 = desc_kmajor_sw32(ring_base + static_cast<uint32_t>(m) * 128u * 32u, 256u, 0u);
-        const uint64_t b_desc0 = desc_kmajor_noswizzle(w_base, (kC3 / 2) * 16u, 128u);
-        uint32_t tap_off[9];
-#pragma unroll
-        for (int tap = 0; tap < 9; ++tap) tap_off[tap] = static_cast<uint32_t>((tap / 3) * g.HP + tap % 3) * 2u;
-        for (int j = 0; next_tile(j) >= 0; ++j, ++lt) {
-          const uint32_t ab = lt & 1u, aph = (lt >> 1) & 1u;
-          mbar_wait_cluster(smem_u32(&bars.acc_empty[ab]), aph ^ 1u);  // both CTAs' epilogues have drained it
-          fence_after();
-          const uint32_t d_tmem = tmem_base + ab * (NM * kC3) + m * kC3;
-#pragma unroll 1
-          for (int kc = 0; kc < 8; ++kc, ++gs) {
-            const uint32_t st = gs % kRingP, ph = (gs / kRingP) & 1u;
-            mbar_wait_cluster(smem_u32(&bars.full[st]), ph);  // both CTAs' slices of this stage have landed
-            fence_after();
-            const uint64_t da_st = a_desc0 + ((st * stage_bytes) >> 4);
-            const uint64_t db_kc = b_desc0 + static_cast<uint32_t>(kc) * (kTapKcBytesP >> 4);
-#pragma unroll
-            for (int tap = 0; tap < 9; ++tap)
-              mma_tf32_pair(d_tmem, da_st + tap_off[tap], db_kc + static_cast<uint32_t>(tap) * (8u * kTapKcBytesP >> 4),
-                            kIdesc, (kc | tap) != 0);
-            commit_pair(smem_u32(&bars.empty[st]));
-          }
-          commit_pair(smem_u32(&bars.acc_full[ab]));
-        }
-      }
-    } else if (m == 0 && lane == 0) {
-      // ======================= relay (peer only): "my slice of stage st is full" -> leader's barrier ==============
-      uint32_t gs = 0;
-      for (int j = 0; next_tile(j) >= 0; ++j) {
-        for (int kc = 0; kc < 8; ++kc, ++gs) {
-          const uint32_t st = gs % kRingP, ph = (gs / kRingP) & 1u;
-          mbar_wait(smem_u32(&bars.full[st]), ph);
-          mbar_arrive_cluster(map_to_cta(smem_u32(&bars.full[st]), 0));
-        }
-      }
-    }
-  } else {
-    // ======================= epilogue (warps 0-3 of both CTAs, each on its own tile) =======================
-    uint32_t lt = 0;
-    const uint32_t t_lane = static_cast<uint32_t>(warp * 32) << 16;
-    for (int j = 0;; ++j, ++lt) {
-      const int tile = next_tile(j);
-      if (tile < 0) break;
-      const bool store = pair_base(j) + rank < total_tiles;
-      const int n = tile / g.tiles_per_img;
-      const int y0 = (tile - n * g.tiles_per_img) * g.R;
-      const uint32_t ab = lt & 1u, aph = (lt >> 1) & 1u;
-      mbar_wait_warp(smem_u32(&bars.acc_full[ab]), aph, lane);
-      fence_after();
-      epilogue_tile<NM, float>(g, n, y0, store, tmem_base + ab * (NM * kC3) + t_lane, s_stage, s_shift, out, tid, 0, 8, 1, [&]() {
-        if (lane == 0) mbar_arrive_cluster(map_to_cta(smem_u32(&bars.acc_empty[ab]), 0));
-      });
-    }
-  }
-
-  fence_before();
-  __syncthreads();
-  cluster_sync_all();  // the peer may still be signalling this CTA's barriers / the leader reading this CTA's ring
-  if (warp == 8) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols));
-}
-
-template <int NM>
-int launch_conv3_pair(const float* x, const float* wpk_pair, const float* shift, float* out, Conv3Geom g,
-                      cudaStream_t stream) {
-  g.halo = (NM * 128 + 2 * g.HP + 2 + 7) & ~7;
-  const size_t smem = kWBytesP + kRingP * (g.halo * 32u) + static_cast<size_t>(g.stage_pos) * kStagePitch * 4 + kC3 * 4 + 256;
-  if (smem + 256u > 232448u) return AFS_ERR_UNSUPPORTED;
-  AFS_CUDA_TRY(cudaFuncSetAttribute(conv3x3_c64_tc_pair_kernel<NM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    static_cast<int>(smem)));
-  const int total = g.N * g.tiles_per_img;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(kNumSMs, 1, 1);
-  cfg.blockDim = dim3(kThreads3, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  // persistent: as many CTA pairs as can be co-resident (a pair that had to wait for a free TPC would run its
-  // whole share of the tiles after everyone else has finished)
-  static int max_pairs[4] = {0, 0, 0, 0};
-  if (max_pairs[NM] == 0) {
-    int n = 0;
-    AFS_CUDA_TRY(cudaOccupancyMaxActiveClusters(&n, conv3x3_c64_tc_pair_kernel<NM>, &cfg));
-    max_pairs[NM] = n > 0 ? n : 1;
-    if (getenv("AFS_DEBUG") != nullptr) fprintf(stderr, "conv3 pair kernel NM=%d: %d co-resident CTA pairs\n", NM, n);
-  }
-  int pairs = (total + 1) / 2;
-  if (pairs > max_pairs[NM]) pairs = max_pairs[NM];
-  cfg.gridDim = dim3(2 * pairs, 1, 1);
-  AFS_CUDA_TRY(cudaLaunchKernelEx(&cfg, conv3x3_c64_tc_pair_kernel<NM>, x, wpk_pair, shift, out, g));
-  AFS_LAUNCH_CHECK();
-  return AFS_OK;
-}
-
 template <int NM, bool BF16, typename TOut, bool EPI2>
 int launch_conv3(const void* x, const void* wpk, const float* shift, TOut* out, Conv3Geom g, cudaStream_t stream) {
   g.halo = (NM * 128 + 2 * g.HP + 2 + 7) & ~7;
@@ -596,24 +404,14 @@ int launch_conv3(const void* x, const void* wpk, const float* shift, TOut* out, 
   return AFS_OK;
 }
 
-// Epilogue groups: AFS_CONV3_EPI2 = 0 / 1 forces one / two groups of four warps; default: two for the bf16 kernel
-// (its MMA phase is half as long), one for the TF32 kernel (MMA-bound; for the large tiles a second staging tile does
-// not fit next to the 144 KB of weights either: the dispatcher falls back to one group when forced).
-inline bool conv3_epi2(bool bf16, int nm) {
-  static const int forced = [] {
-    const char* e = getenv("AFS_CONV3_EPI2");
-    return e == nullptr ? -1 : (e[0] == '1' ? 1 : 0);
-  }();
-  // measured: two groups do not help the TF32 kernel even where they fit (block 3, two accumulators: 0.155 ms with,
-  // 0.144 ms without) -- it is MMA-bound at every tile size
-  (void)nm;
-  return forced < 0 ? bf16 : forced == 1;
-}
-
+// Epilogue groups: two for the bf16 kernel (its MMA phase is half as long), one for the TF32 kernel.  The TF32 kernel
+// is MMA-bound at every tile size: measured, two groups do not help it even where they fit (block 3, two
+// accumulators: 0.155 ms with, 0.144 ms without), and for the large tiles a second staging tile does not fit next to
+// its 144 KB of weights.
 template <bool BF16, typename TOut>
 int dispatch_conv3(int NM, const void* x, const void* wpk, const float* shift, TOut* out, const Conv3Geom& g,
                    cudaStream_t stream) {
-  if (conv3_epi2(BF16, NM)) {
+  if constexpr (BF16) {
     int rc;
     switch (NM) {
       case 1: rc = launch_conv3<1, BF16, TOut, true>(x, wpk, shift, out, g, stream); break;
@@ -662,15 +460,11 @@ int conv3_acc_tiles(const Conv3Geom& g) {
   return total;
 }
 
-// Geometry with the accumulator count that needs the fewest MMAs (AFS_CONV3_NM4 = 0 / 1 forces three / tries four).
+// Geometry with the accumulator count (three or four) that needs the fewest MMAs.
 int conv3_best_geometry(int32_t N, int32_t H, int32_t Wd, float negative_slope, int32_t pool3, Conv3Geom* gp) {
-  static const int forced = [] {
-    const char* e = getenv("AFS_CONV3_NM4");
-    return e == nullptr ? -1 : (e[0] == '1' ? 1 : 0);
-  }();
   Conv3Geom g3, g4;
   const int nm3 = conv3_geometry(N, H, Wd, negative_slope, pool3, 3, &g3);
-  if (nm3 < 0 || forced == 0) {
+  if (nm3 < 0) {
     *gp = g3;
     return nm3;
   }
@@ -682,12 +476,6 @@ int conv3_best_geometry(int32_t N, int32_t H, int32_t Wd, float negative_slope, 
   *gp = g3;
   return nm3;
 }
-
-// 0: one CTA per SM (default).  1: CTA pairs (cta_group::2).  Initialised from AFS_CONV3_PAIR.
-std::atomic<int> g_pair_mode{[] {
-  const char* e = getenv("AFS_CONV3_PAIR");
-  return (e != nullptr && e[0] == '1') ? 1 : 0;
-}()};
 
 inline uint16_t round_bf16_host(float v) {  // round to nearest even (what __float2bfloat16_rn does); NaN kept quiet
   uint32_t b;
@@ -709,12 +497,7 @@ inline float round_tf32_host(float v) {  // cvt.rna.tf32.f32: nearest, ties away
 }  // namespace
 }  // namespace afs
 
-extern "C" int afs_conv3x3_c64_set_pair_mode(int32_t on) {
-  afs::g_pair_mode.store(on ? 1 : 0, std::memory_order_relaxed);
-  return AFS_OK;
-}
-
-extern "C" size_t afs_conv3x3_c64_packed_floats(void) { return 2 * (afs::kWBytes3 / 4); }
+extern "C" size_t afs_conv3x3_c64_packed_floats(void) { return afs::kWBytes3 / 4; }
 
 extern "C" int afs_conv3x3_c64_pack_weights(const float* w_folded_host, float* packed_host) {
   using namespace afs;
@@ -728,8 +511,6 @@ extern "C" int afs_conv3x3_c64_pack_weights(const float* w_folded_host, float* p
             const int ci = 8 * kc + 4 * ch + i;
             const float v = round_tf32_host(w_folded_host[(co * kC3 + ci) * 9 + tap]);
             packed_host[(((tap * 8 + kc) * 2 + ch) * kC3 + co) * 4 + i] = v;
-            // second copy for the CTA-pair kernel: [rank = co / 32][tap][kc][chunk][co % 32][4]
-            packed_host[kWBytes3 / 4 + ((((co / 32) * 9 + tap) * 8 + kc) * 2 + ch) * (kC3 / 2) * 4 + (co % 32) * 4 + i] = v;
           }
   return AFS_OK;
 }
@@ -747,18 +528,9 @@ extern "C" int afs_conv3x3_c64_bn_act_fwd_tf32(const float* x, int32_t N, int32_
   if (Wd > 61) return AFS_ERR_UNSUPPORTED;  // the operand ring of wider rows does not fit next to the weights
   if (N == 0) return AFS_OK;
   Conv3Geom g;
-  int NM = conv3_geometry(N, H, Wd, negative_slope, pool3, 3, &g);
+  int NM = conv3_best_geometry(N, H, Wd, negative_slope, pool3, &g);
   if (NM < 0) return NM;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (g_pair_mode.load(std::memory_order_relaxed) != 0 && static_cast<int64_t>(N) * g.tiles_per_img >= 2) {
-    const float* w_pair = w_packed + kWBytes3 / 4;
-    switch (NM) {
-      case 1: return launch_conv3_pair<1>(x, w_pair, shift, out, g, stream);
-      case 2: return launch_conv3_pair<2>(x, w_pair, shift, out, g, stream);
-      default: return launch_conv3_pair<3>(x, w_pair, shift, out, g, stream);
-    }
-  }
-  NM = conv3_best_geometry(N, H, Wd, negative_slope, pool3, &g);
   int rc = dispatch_conv3<false, float>(NM, x, w_packed, shift, out, g, stream);
   if (rc == AFS_ERR_UNSUPPORTED && NM == 4) {  // no shared memory for four accumulators' stages: three
     NM = conv3_geometry(N, H, Wd, negative_slope, pool3, 3, &g);

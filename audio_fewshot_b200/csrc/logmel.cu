@@ -267,7 +267,6 @@ extern "C" int afs_logmel_plan_create(const afs_logmel_cfg* cfg, const float* fb
   plan->nnz = static_cast<int>(weights.size());
   plan->d_window = nullptr; plan->d_tw1024 = nullptr; plan->d_band = nullptr; plan->d_weights = nullptr;
   plan->d_band64 = nullptr; plan->d_weights64 = nullptr;
-  plan->d_tc = nullptr;
   plan->engine = AFS_LOGMEL_ENGINE_AUTO;
 
   int prev = 0;
@@ -291,7 +290,6 @@ extern "C" int afs_logmel_plan_create(const afs_logmel_cfg* cfg, const float* fb
   if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_kernel<true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_kernel<true, int16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e == cudaSuccess) e = logmel::pair_prepare();
-  if (e == cudaSuccess && logmel::tc_tables_create(plan, fb_host) != AFS_OK) e = cudaErrorMemoryAllocation;
   cudaSetDevice(prev);
   if (e != cudaSuccess) {
     afs_logmel_plan_destroy(plan);
@@ -309,14 +307,14 @@ extern "C" int afs_logmel_plan_destroy(afs_logmel_plan* plan) {
   cudaFree(plan->d_weights);
   cudaFree(plan->d_band64);
   cudaFree(plan->d_weights64);
-  afs::logmel::tc_tables_destroy(plan);
   delete plan;
   return AFS_OK;
 }
 
 extern "C" int afs_logmel_plan_set_engine(afs_logmel_plan* plan, int32_t engine) {
-  if (plan == nullptr || (engine < AFS_LOGMEL_ENGINE_FFT || engine > AFS_LOGMEL_ENGINE_AUTO)) return AFS_ERR_INVALID_ARG;
-  if (engine == AFS_LOGMEL_ENGINE_TC && plan->d_tc == nullptr) return AFS_ERR_UNSUPPORTED;
+  if (plan == nullptr ||
+      (engine != AFS_LOGMEL_ENGINE_FFT && engine != AFS_LOGMEL_ENGINE_PAIR && engine != AFS_LOGMEL_ENGINE_AUTO))
+    return AFS_ERR_INVALID_ARG;
   plan->engine = engine;
   return AFS_OK;
 }
@@ -365,7 +363,6 @@ int logmel_launch(const afs_logmel_plan* plan, const S* wav, float pcm_scale, in
     p.noise_lo = aug->noise_std_lo; p.noise_hi = aug->noise_std_hi;
     p.max_shift = aug->max_shift;
   }
-  if (plan->engine == AFS_LOGMEL_ENGINE_TC) return logmel::tc_launch<S>(plan, p, aug != nullptr, stream);
   if (plan->engine == AFS_LOGMEL_ENGINE_PAIR || (plan->engine == AFS_LOGMEL_ENGINE_AUTO && aug == nullptr))
     return logmel::pair_launch<S>(plan, p, aug != nullptr, stream);
   if (aug != nullptr) {

@@ -1,6 +1,6 @@
-// Shared by the two engines of the fused waveform -> log-mel front-end (logmel.cu: radix-8 FFT on the FMA pipe;
-// logmel_tc.cu: four-step DFT on tcgen05): the plan, the kernel parameters, and the sample fetch with the Philox
-// waveform augmentation.
+// Shared by the two engines of the fused waveform -> log-mel front-end (logmel.cu: radix-8 FFT, one frame per 64
+// threads; logmel_pair.cu: two frames per warp as one 1024-point FFT): the plan, the kernel parameters, and the sample
+// fetch with the Philox waveform augmentation.
 #pragma once
 #include <stdint.h>
 
@@ -19,7 +19,6 @@ struct afs_logmel_plan {
   float* d_weights;  // [nnz]
   int* d_band64;     // the same table with start shifts chosen for 64-bit power reads (pair engine)
   float* d_weights64;
-  void* d_tc;        // tensor-core engine: DFT operand images + twiddle table (logmel_tc.cu); null when unsupported
 };
 
 namespace afs {
@@ -129,12 +128,6 @@ inline int num_frames(const afs_logmel_cfg& cfg, int64_t L) {
   if (L < cfg.n_fft) return 0;
   return static_cast<int>(1 + (L - cfg.n_fft) / cfg.hop);
 }
-
-// logmel_tc.cu
-int tc_tables_create(afs_logmel_plan* plan, const float* fb_host);  // sets plan->d_tc (or leaves it null)
-void tc_tables_destroy(afs_logmel_plan* plan);
-template <typename S>
-int tc_launch(const afs_logmel_plan* plan, const Params& p, bool aug, cudaStream_t stream);
 
 // logmel_pair.cu
 cudaError_t pair_prepare();

@@ -58,8 +58,8 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
 }
 
 // The same wait with a suspend-time hint: the thread sleeps in hardware until the phase completes (or the hint, in
-// ns, runs out) instead of re-issuing try_wait -- for kernels in which many warps wait at once (logmel_tc.cu: without
-// the hint the polling lanes were 65 % of all executed instructions).
+// ns, runs out) instead of re-issuing try_wait -- for kernels in which many warps wait at once (measured on a 16-warp
+// tcgen05 log-mel kernel: without the hint the polling lanes were 65 % of all executed instructions).
 __device__ __forceinline__ void mbar_wait_sleep(uint32_t bar, uint32_t parity) {
   asm volatile(
       "{\n\t"
@@ -200,86 +200,7 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
       : "r"(taddr));
 }
 
-// 4 consecutive accumulator columns of this thread's TMEM lane (no wait: pair with tmem_wait_ld)
-__device__ __forceinline__ void tmem_ld4(uint32_t taddr, uint32_t (&v)[4]) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3])
-               : "r"(taddr));
-}
-
-// 16 consecutive accumulator columns of this thread's TMEM lane (no wait: pair with tmem_wait_ld)
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-        "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-      : "r"(taddr));
-}
-
-// ---- CTA pairs (thread-block clusters of 2, tcgen05 cta_group::2)
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t map_to_cta(uint32_t smem_addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {  // acquire at cluster scope
-  asm volatile(
-      "{\n\t"
-      ".reg .pred P1;\n\t"
-      "LAB_WAIT:\n\t"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P1, [%0], %1;\n\t"
-      "@P1 bra DONE;\n\t"
-      "bra LAB_WAIT;\n\t"
-      "DONE:\n\t"
-      "}" ::"r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void mma_tf32_pair(uint32_t d_tmem, uint64_t da, uint64_t db, uint32_t idesc, bool accumulate) {
-  const uint32_t acc = accumulate ? 1u : 0u;
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n\t"
-      "}\n" ::"r"(d_tmem), "l"(da), "l"(db), "r"(idesc), "r"(acc)
-      : "memory");
-}
-__device__ __forceinline__ void commit_pair(uint32_t bar) {  // arrives on the same barrier of both CTAs
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-               "h"(static_cast<uint16_t>(3))
-               : "memory");
-}
-
-// ---- kind::f16 (fp16 operands, fp32 accumulate) with either operand major
-// a_mn / b_mn = 1: the operand is MN-major (M or N contiguous in shared memory), 0: K-major.
-__host__ __device__ constexpr uint32_t idesc_f16(int M, int N, int a_mn, int b_mn) {
-  return (1u << 4) | (static_cast<uint32_t>(a_mn) << 15) | (static_cast<uint32_t>(b_mn) << 16) |
-         (static_cast<uint32_t>(N >> 3) << 17) | (static_cast<uint32_t>(M >> 4) << 24);
-}
-// Generic shared-memory matrix descriptor: layout 0 = no swizzle, 6 = 32 B, 4 = 64 B, 2 = 128 B.
-//   K-major,  no swizzle: LBO = distance between the 8-element K groups, SBO = between 8-row groups
-//   MN-major, no swizzle: LBO = distance between the 8-row K groups,    SBO = between 8-element MN groups
-//   MN-major, swizzled:   LBO = distance between MN groups of one swizzle row (32 elements for 64 B), SBO = between
-//                         8-row K groups (both orders measured on B200: tools/tc_dft_probe.cu)
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo, uint32_t layout) {
-  uint64_t d = static_cast<uint64_t>((saddr >> 4) & 0x3FFFu);
-  d |= static_cast<uint64_t>((lbo >> 4) & 0x3FFFu) << 16;
-  d |= static_cast<uint64_t>((sbo >> 4) & 0x3FFFu) << 32;
-  d |= static_cast<uint64_t>(1) << 46;
-  d |= static_cast<uint64_t>(layout) << 61;
-  return d;
-}
+// ---- kind::f16 (16-bit operands, fp32 accumulate; the caller's instruction descriptor selects fp16 or bf16)
 __device__ __forceinline__ void mma_f16(uint32_t d_tmem, uint64_t da, uint64_t db, uint32_t idesc, bool accumulate) {
   const uint32_t acc = accumulate ? 1u : 0u;
   asm volatile(

@@ -45,7 +45,7 @@ def _need_cuda(t, name, dtype=torch.float32):
 class LogMelPlan:
     """Owns an afs_logmel_plan (device tables: window, twiddles, packed mel bands)."""
 
-    ENGINES = {"fft": 0, "tc": 1, "pair": 2, "auto": 3}
+    ENGINES = {"fft": 0, "pair": 2, "auto": 3}
 
     def __init__(self, fb, window, hop, n_mels, center=True, log_mult=10.0, log_eps=2.220446049250313e-16,
                  device=None, engine=None):
@@ -72,8 +72,10 @@ class LogMelPlan:
             self.set_engine(engine)
 
     def set_engine(self, engine):
-        """"pair": two frames per warp as one 1024-point complex FFT; "fft": one frame per 64 threads, radix-8; "tc":
-        four-step DFT on the tcgen05 tensor cores; "auto" (default): "pair", "fft" for augmented launches."""
+        """"pair": two frames per warp as one 1024-point complex FFT; "fft": one frame per 64 threads, radix-8;
+        "auto" (default): "pair", "fft" for augmented launches.  Any other name raises ValueError."""
+        if engine not in self.ENGINES:
+            raise ValueError("unknown log-mel engine %r; expected one of %s" % (engine, sorted(self.ENGINES)))
         _lib.check(_lib.lib().afs_logmel_plan_set_engine(self._handle, self.ENGINES[engine]), "afs_logmel_plan_set_engine")
         self.engine = engine
 
@@ -232,12 +234,6 @@ def conv3x3_c64_pack_weights(w_folded):
     _lib.check(h.afs_conv3x3_c64_pack_weights(w.ctypes.data_as(C.c_void_p), packed.ctypes.data_as(C.c_void_p)),
                "afs_conv3x3_c64_pack_weights")
     return packed
-
-
-def conv3x3_c64_set_pair_mode(on):
-    """Process-wide switch between the one-CTA-per-SM kernel (default) and the CTA-pair (cta_group::2) variant of
-    conv3x3_c64_bn_act; results are bit-identical."""
-    _lib.check(_lib.lib().afs_conv3x3_c64_set_pair_mode(1 if on else 0), "afs_conv3x3_c64_set_pair_mode")
 
 
 def conv3x3_c64_supported(x):

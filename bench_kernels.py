@@ -62,7 +62,7 @@ def main():
     for tag, L, hop, B in (("S5 L=80000 hop=512", 80000, 512, 800), ("S5 L=80000 hop=512", 80000, 512, 3200),
                            ("S1 L=16000 hop=102", 16000, 102, 800)):
         for engine, kname in (("pair", "logmel_pair_kernel<false> (warp-per-frame-pair engine, default)"),
-                              ("fft", "logmel_kernel<false> (radix-8 engine)"), ("tc", "logmel_tc_kernel<false> (tcgen05 DFT engine)")):
+                              ("fft", "logmel_kernel<false> (radix-8 engine)")):
             fr = LogMelFrontEnd(hop_length=hop, n_mels=128, mean=-15.0, std=26.0, engine=engine).to(dev).eval()
             wav = torch.randn(B, L, device=dev) * 0.1
             T = 1 + L // hop

@@ -89,18 +89,15 @@ typedef struct afs_logmel_plan afs_logmel_plan; /* opaque; owns device tables */
 int afs_logmel_plan_create(const afs_logmel_cfg* cfg, const float* fb_host,
                            const float* window_host, int device, afs_logmel_plan** plan_out);
 int afs_logmel_plan_destroy(afs_logmel_plan* plan);
-/* Three engines compute the same features (each within the 1e-4 dB tolerance of the float64 spec):
+/* Two engines compute the same features (each within the 1e-4 dB tolerance of the float64 spec):
  *   AFS_LOGMEL_ENGINE_FFT   one frame per 64 threads: 512-point complex radix-8 FFT in registers on the FMA pipe
  *                           (packed-f32x2 arithmetic), three shared-memory exchanges per frame, csrc/logmel.cu
- *   AFS_LOGMEL_ENGINE_TC    four-step 32x32 DFT as tcgen05 GEMMs (fp16 hi/lo operand pairs, fp32 accumulators in
- *                           tensor memory), csrc/logmel_tc.cu
  *   AFS_LOGMEL_ENGINE_PAIR  two frames per warp as ONE 1024-point complex FFT (32 x 32 in registers): one exchange per
  *                           frame pair, in-warp shuffle split, csrc/logmel_pair.cu -- the fastest for plain launches
  *   AFS_LOGMEL_ENGINE_AUTO  (default) PAIR, except FFT when waveform augmentation is requested (its Philox draws are
  *                           shared by sample pairs there)
- * AFS_ERR_UNSUPPORTED when the plan cannot run the requested engine.                                       */
+ * The numbering is part of the ABI and has a gap at 1; any other value returns AFS_ERR_INVALID_ARG.          */
 #define AFS_LOGMEL_ENGINE_FFT 0
-#define AFS_LOGMEL_ENGINE_TC 1
 #define AFS_LOGMEL_ENGINE_PAIR 2
 #define AFS_LOGMEL_ENGINE_AUTO 3
 int afs_logmel_plan_set_engine(afs_logmel_plan* plan, int32_t engine);
@@ -178,17 +175,13 @@ int afs_conv1_train_bwd(const float* x, const float* grad_out, int32_t N, int32_
  * Replaces layer2..layer4 of libfewshot_core/model/backbone/conv_four.py:67-86,104-113 in eval mode.
  * x [N, H, Wd, 64] fp32 NHWC (device); out [N, H, Wd, 64] or, pooled, [N, H/3, Wd/3, 64] NHWC (device).
  * w_packed (device, afs_conv3x3_c64_packed_floats() floats, 16-byte aligned): the BatchNorm-folded weights in
- * operand order (once for the one-CTA kernel, once split in halves for the CTA-pair kernel), produced on the host by afs_conv3x3_c64_pack_weights from w_folded_host [64][64][3][3] (OIHW)
- * with round-to-nearest TF32; shift [64] (device) = (bias - mean)*gamma/sqrt(var+eps) + beta.
+ * operand order [tap][8-channel group][4-channel chunk][cout][4], produced on the host by afs_conv3x3_c64_pack_weights
+ * from w_folded_host [64][64][3][3] (OIHW) with round-to-nearest TF32;
+ * shift [64] (device) = (bias - mean)*gamma/sqrt(var+eps) + beta.
  * Built for Wd <= 61; AFS_ERR_UNSUPPORTED otherwise (the caller keeps cuDNN for such shapes).
- * Tiling is chosen per shape (three or four 128-row accumulators per tile, whichever needs fewer MMAs); the
- * development switches AFS_CONV3_NM4=0 (always three) and AFS_CONV3_EPI2=0/1 (one / two epilogue groups) in the
- * environment select the measured alternatives; results are bit-identical across them.                       */
+ * Tiling is chosen per shape: three or four 128-row accumulators per tile, whichever needs fewer MMAs (three when
+ * the operand ring of four does not fit in shared memory).                                                    */
 size_t afs_conv3x3_c64_packed_floats(void);
-/* Kernel variant switch (process-wide; default 0, or 1 when AFS_CONV3_PAIR=1 is in the environment): 1 runs the block
- * on CTA pairs (thread-block clusters of 2, tcgen05 cta_group::2: each CTA keeps half of the weights).  Results are
- * bit-identical; on B200 the pair variant is not faster (DESIGN.md 3.2), it is kept as the measured alternative.   */
-int afs_conv3x3_c64_set_pair_mode(int32_t on);
 int afs_conv3x3_c64_pack_weights(const float* w_folded_host, float* packed_host);
 int afs_conv3x3_c64_bn_act_fwd_tf32(const float* x, int32_t N, int32_t H, int32_t Wd, const float* w_packed,
                                     const float* shift, float negative_slope, int32_t pool3, float* out,

@@ -90,10 +90,10 @@ def test_header_is_plain_c_and_a_c_host_links(tmp_path):
     assert out.stdout.split() == ["workspace", "too", "small", str(len(names))]
 
 
-def test_conv3x3_weight_packing_layouts_and_tf32_rounding():
-    """afs_conv3x3_c64_pack_weights is host code: check on the CPU that both operand layouts hold the weights where
-    the kernels expect them -- one-CTA kernel [tap][kc][chunk][cout][4], CTA-pair kernel [cout/32][tap][kc][chunk]
-    [cout%32][4] -- and that values are rounded to the nearest TF32 (ties away from zero, what cvt.rna.tf32 does)."""
+def test_conv3x3_weight_packing_layout_and_tf32_rounding():
+    """afs_conv3x3_c64_pack_weights is host code: check on the CPU that the operand layout holds the weights where
+    the kernel expects them -- [tap][kc][chunk][cout][4] -- and that values are rounded to the nearest TF32 (ties away
+    from zero, what cvt.rna.tf32 does)."""
     import numpy as np
     from audio_fewshot_b200 import _lib
     h = _lib.lib()
@@ -101,17 +101,14 @@ def test_conv3x3_weight_packing_layouts_and_tf32_rounding():
     w = (rng.standard_normal((64, 64, 3, 3)) * 0.1).astype(np.float32)
     w[0, 0, 0, 0] = np.float32(1.0) + np.float32(2.0 ** -11)  # exactly half a TF32 ulp above 1: rounds away from zero
     n = int(h.afs_conv3x3_c64_packed_floats())
-    assert n == 2 * 9 * 8 * 2 * 64 * 4
+    assert n == 9 * 8 * 2 * 64 * 4
     packed = np.empty(n, np.float32)
     assert h.afs_conv3x3_c64_pack_weights(w.ctypes.data_as(ctypes.c_void_p), packed.ctypes.data_as(ctypes.c_void_p)) == 0
     bits = w.view(np.uint32).astype(np.uint64)
     want = (((bits + 0x1000) & ~np.uint64(0x1FFF)).astype(np.uint32)).view(np.float32)  # [co][ci][ky][kx]
     assert want[0, 0, 0, 0] == np.float32(1.0) + np.float32(2.0 ** -10)
-    single = packed[: n // 2].reshape(9, 8, 2, 64, 4)      # [tap][kc][chunk][cout][i]
-    pair = packed[n // 2:].reshape(2, 9, 8, 2, 32, 4)       # [rank][tap][kc][chunk][cout % 32][i]
     ref = want.reshape(64, 8, 2, 4, 9)                      # [co][kc][chunk][i][tap]  (ci = 8 kc + 4 chunk + i)
-    assert np.array_equal(single, ref.transpose(4, 1, 2, 0, 3))
-    assert np.array_equal(pair, ref.reshape(2, 32, 8, 2, 4, 9).transpose(0, 5, 2, 3, 1, 4))
+    assert np.array_equal(packed.reshape(9, 8, 2, 64, 4), ref.transpose(4, 1, 2, 0, 3))  # [tap][kc][chunk][cout][i]
     assert h.afs_conv3x3_c64_pack_weights(None, packed.ctypes.data_as(ctypes.c_void_p)) == -1
 
 

@@ -1,4 +1,4 @@
-// Hardware probe for the tensor-core DFT log-mel kernel (development tool, B200 / sm_100a).
+// Hardware probe for a tensor-core DFT log-mel kernel (development tool, B200 / sm_100a; DESIGN.md 3.1b, 9).
 //
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -I audio_fewshot_b200/csrc \
 //        tools/tc_dft_probe.cu -o tools/tc_dft_probe && ./tools/tc_dft_probe
@@ -36,6 +36,11 @@ __host__ __device__ constexpr uint32_t idesc_f16(int M, int N, int a_mn, int b_m
          (static_cast<uint32_t>(N >> 3) << 17) | (static_cast<uint32_t>(M >> 4) << 24);
 }
 
+// Generic shared-memory matrix descriptor: layout 0 = no swizzle, 6 = 32 B, 4 = 64 B, 2 = 128 B.
+//   K-major,  no swizzle: LBO = distance between the 8-element K groups, SBO = between 8-row groups
+//   MN-major, no swizzle: LBO = distance between the 8-row K groups,    SBO = between 8-element MN groups
+//   MN-major, swizzled:   LBO = distance between MN groups of one swizzle row (32 elements for 64 B), SBO = between
+//                         8-row K groups (both orders measured on B200 with this probe)
 __device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo, uint32_t layout) {
   uint64_t d = static_cast<uint64_t>((saddr >> 4) & 0x3FFFu);
   d |= static_cast<uint64_t>((lbo >> 4) & 0x3FFFu) << 16;
@@ -43,17 +48,6 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo, uint
   d |= static_cast<uint64_t>(1) << 46;
   d |= static_cast<uint64_t>(layout) << 61;
   return d;
-}
-
-__device__ __forceinline__ void mma_f16(uint32_t d_tmem, uint64_t da, uint64_t db, uint32_t idesc, bool accumulate) {
-  const uint32_t acc = accumulate ? 1u : 0u;
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
-      "}\n" ::"r"(d_tmem), "l"(da), "l"(db), "r"(idesc), "r"(acc)
-      : "memory");
 }
 
 constexpr int kHop = 512;

@@ -1,5 +1,5 @@
 """Bring-up check of the warp-per-frame-pair log-mel engine (csrc/logmel_pair.cu) on a B200: features against the float64
-spec and the radix-8 engine, and the engines' times (AFS_PAIR_VARIANT selects the prefetch point at plan creation).
+spec and the radix-8 engine, and the engines' times.
     python tools/try_logmel_pair.py [--quick]"""
 import os
 import sys
@@ -44,7 +44,6 @@ def timeit(fr, wav, out, flush):
 
 
 if __name__ == "__main__":
-    print("AFS_PAIR_MODE=%s" % os.environ.get("AFS_PAIR_MODE", "0"))
     check(1, 80000, 512)
     check(3, 80000, 512)
     check(2, 16000, 102)
