@@ -26,11 +26,19 @@ namespace {
 
 constexpr int kCT = 64;            // output channels
 constexpr int kAcStats = 54;       // 9 sums + 45 products (upper triangle of R, row-major)
+constexpr int kAcCols = kAcStats + 1;  // a partial row: the 54 sums, then the pivot they were taken around
 constexpr int kBwdStats = 11;      // per channel: A1, A2, G[9]
 
 // ------------------------------------------------------------------------------------------------ autocorrelation
+// The sums are taken of x_t - p for a pivot p near the mean of the input (zero-padded taps included, as -p): with a DC
+// offset (normalised log-mel in silence sits near -5.4; an unnormalised input may sit anywhere) the sums of raw
+// products are dominated by mean^2 and lose the variance to fp32 rounding, while the centred moments that BatchNorm
+// needs are the same for x_t - p.  p is the mean of 32 inputs spread over the batch: every warp loads the same 32
+// values and reduces them in the same butterfly, so every thread holds the same p.
 __global__ void __launch_bounds__(256)
 conv1_autocorr_kernel(const float* __restrict__ x, int64_t total, int H, int W, float* __restrict__ partials) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const float pivot = total > 0 ? warp_sum(__ldg(x + total * lane / 32)) * (1.f / 32.f) : 0.f;
   float acc[kAcStats];
 #pragma unroll
   for (int i = 0; i < kAcStats; ++i) acc[i] = 0.f;
@@ -47,7 +55,7 @@ conv1_autocorr_kernel(const float* __restrict__ x, int64_t total, int H, int W, 
 #pragma unroll
       for (int dx = 0; dx < 3; ++dx) {
         const int yy = y + dy - 1, xc = xx + dx - 1;
-        v[dy * 3 + dx] = (yy >= 0 && yy < H && xc >= 0 && xc < W) ? __ldg(img + static_cast<int64_t>(yy) * W + xc) : 0.f;
+        v[dy * 3 + dx] = ((yy >= 0 && yy < H && xc >= 0 && xc < W) ? __ldg(img + static_cast<int64_t>(yy) * W + xc) : 0.f) - pivot;
       }
     }
     int k = 9;
@@ -62,7 +70,6 @@ conv1_autocorr_kernel(const float* __restrict__ x, int64_t total, int H, int W, 
     }
   }
   __shared__ float s_red[8][kAcStats];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
   for (int i = 0; i < kAcStats; ++i) {
     const float v = warp_sum(acc[i]);
@@ -73,7 +80,9 @@ conv1_autocorr_kernel(const float* __restrict__ x, int64_t total, int H, int W, 
     float v = 0.f;
 #pragma unroll
     for (int w = 0; w < 8; ++w) v += s_red[w][threadIdx.x];
-    partials[static_cast<int64_t>(blockIdx.x) * kAcStats + threadIdx.x] = v;
+    partials[static_cast<int64_t>(blockIdx.x) * kAcCols + threadIdx.x] = v;
+  } else if (threadIdx.x == kAcStats) {
+    partials[static_cast<int64_t>(blockIdx.x) * kAcCols + kAcStats] = pivot;
   }
 }
 
@@ -266,7 +275,9 @@ conv1_train_bwd_kernel(const float* __restrict__ x, const float* __restrict__ g,
 // ------------------------------------------------------------------------------------------------ finalisers
 // One CTA of 64 threads (thread = channel) turns the autocorrelation partials into everything the forward and the
 // backward kernels need, in fp64: s[9], R[9][9] (kept for the backward), mean_nob, invstd, scale, shift, and the
-// running-statistics update of nn.BatchNorm2d.  stats layout (doubles): [0,9) s, [9,90) R row-major.
+// running-statistics update of nn.BatchNorm2d.  stats layout (doubles): [0,9) s, [9,90) R row-major.  The partials
+// are sums of x_t - p; the variance is taken from their centred moments (which p does not change), s and R are
+// shifted back in fp64: s[t] = s'[t] + p P, R[t,u] = R'[t,u] + p (s'[t] + s'[u]) + p^2 P.
 __global__ void __launch_bounds__(64)
 conv1_train_stats_kernel(const float* __restrict__ partials, int n_part, double P, const float* __restrict__ w,
                          const float* __restrict__ bias, const float* __restrict__ gamma,
@@ -275,37 +286,43 @@ conv1_train_stats_kernel(const float* __restrict__ partials, int n_part, double 
                          float* __restrict__ invstd, float* __restrict__ scale, float* __restrict__ shift) {
   __shared__ double s_st[kAcStats];
   __shared__ double s_R[81];
+  __shared__ double s_cov[81];
   const int c = threadIdx.x;
   if (c < kAcStats) {
     double v = 0.0;
-    for (int i = 0; i < n_part; ++i) v += static_cast<double>(partials[static_cast<int64_t>(i) * kAcStats + c]);
+    for (int i = 0; i < n_part; ++i) v += static_cast<double>(partials[static_cast<int64_t>(i) * kAcCols + c]);
     s_st[c] = v;
   }
   __syncthreads();
+  const double p = static_cast<double>(partials[kAcStats]);  // every row carries the same pivot
   if (c == 0) {
     int k = 9;
     for (int t = 0; t < 9; ++t)
       for (int u = t; u < 9; ++u) {
-        s_R[t * 9 + u] = s_st[k];
-        s_R[u * 9 + t] = s_st[k];
+        const double r = s_st[k] + p * (s_st[t] + s_st[u]) + p * p * P;
+        const double cv = s_st[k] / P - s_st[t] * s_st[u] / (P * P);
+        s_R[t * 9 + u] = r;
+        s_R[u * 9 + t] = r;
+        s_cov[t * 9 + u] = cv;
+        s_cov[u * 9 + t] = cv;
         ++k;
       }
   }
   __syncthreads();
-  if (c < 9) stats[c] = s_st[c];
+  if (c < 9) stats[c] = s_st[c] + p * P;
   for (int i = c; i < 81; i += 64) stats[9 + i] = s_R[i];
   double wc[9], m = 0.0;
 #pragma unroll
   for (int t = 0; t < 9; ++t) {
     wc[t] = static_cast<double>(w[c * 9 + t]);
-    m += wc[t] * s_st[t];
+    m += wc[t] * (s_st[t] + p * P);
   }
   m /= P;  // mean of the conv output without its bias
   double var = 0.0;
 #pragma unroll
   for (int t = 0; t < 9; ++t)
 #pragma unroll
-    for (int u = 0; u < 9; ++u) var += wc[t] * wc[u] * (s_R[t * 9 + u] / P - s_st[t] * s_st[u] / (P * P));
+    for (int u = 0; u < 9; ++u) var += wc[t] * wc[u] * s_cov[t * 9 + u];
   if (var < 0.0) var = 0.0;
   const double is = 1.0 / sqrt(var + eps);
   const double sc = static_cast<double>(gamma[c]) * is;

@@ -167,7 +167,7 @@ class _Conv1TrainFn(torch.autograd.Function):
         x = x.contiguous()
         dev = x.device
         f32 = dict(dtype=torch.float32, device=dev)
-        ac = torch.empty((int(h.afs_conv1_train_num_partials(0)), 54), **f32)
+        ac = torch.empty((int(h.afs_conv1_train_num_partials(0)), 55), **f32)
         _lib.check(h.afs_conv1_autocorr(_ptr(x), N, H, Wd, _ptr(ac), _stream()), "afs_conv1_autocorr")
         w32 = weight.detach().reshape(64, 9).contiguous()
         b32, g32, be32 = bias.detach().contiguous(), gamma.detach().contiguous(), beta.detach().contiguous()

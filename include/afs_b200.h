@@ -143,8 +143,10 @@ int afs_conv1_bn_act_pool3_fwd_tf32(const float* x, int32_t N, int32_t H, int32_
  * layer1 of libfewshot_core/model/backbone/conv_four.py:61-66 under set_forward_loss.  The block has one input
  * channel, so the BatchNorm statistics and the dense BatchNorm-backward correction terms are functions of the 9-tap
  * sums s[t] and the 9x9 autocorrelation R[t,u] of the input (csrc/conv1_train.cu).  All pointers are device pointers.
- *   afs_conv1_autocorr: x [N,1,H,Wd] -> partials [afs_conv1_train_num_partials(0)][54] (9 sums, then the upper
- *     triangle of R row-major); the caller adds the rows (fixed order: deterministic).
+ *   afs_conv1_autocorr: x [N,1,H,Wd] -> partials [afs_conv1_train_num_partials(0)][55]: 9 sums, then the upper
+ *     triangle of R row-major, of the tap values minus a pivot p near the input's mean (so that a DC offset does not
+ *     cancel the variance away in fp32), then p, the same in every row; afs_conv1_train_stats adds the rows in a
+ *     fixed order (deterministic) and shifts s and R back in fp64.
  *   afs_conv1_train_fwd: out[N, H/3, Wd/3, 64] (NHWC) = MaxPool3(act(scale_c * (w_c * x) + shift_c)); w [64*9] raw
  *     conv weights, scale = gamma*invstd, shift = beta - mean_nob*scale (the conv bias cancels under batch statistics).
  *   afs_conv1_train_bwd: grad_out [N, H/3, Wd/3, 64] (NHWC) -> partials [afs_conv1_train_num_partials(1)][64][11]:
