@@ -21,17 +21,29 @@
 //                     of four 24 KB operand buffers
 //   EPI   warps 4-11  thread = (pooled pixel, 32-channel half): the three windows of a row with three tcgen05.ld behind
 //                     one wait, accumulators handed back, FMNMX3 folds into the running max, + folded shift,
-//                     activation, warp transpose through a padded staging tile so that every store instruction writes
-//                     whole 128-byte half-rows of the NHWC output (64-byte half-rows of the bf16 output)
+//                     activation; each thread writes its pixel's 32 channels into the warp's staging box (32 pixels x
+//                     32 channels, the TMA swizzle applied: 128-byte rows, 64-byte for the bf16 output) and one lane
+//                     stores the box with a TMA tensor store.  Two boxes per warp, so a tile's store drains while the
+//                     next tile is folded; TMA drops the rows of a tail tile past the last pixel.
 //   MMA   warp 12     one thread: per window row 2 tcgen05.mma M128 N192 K8 (TF32) into one of two 192-column
 //                     accumulator sets; tcgen05.commit hands accumulators to the epilogue and operand buffers back
 //                     to BUILD
 // Measured on B200, 3 200 clips (profiles/r02_conv1_tc_variants.txt): round-1 kernel 1.08 ms; warp-specialised with
 // per-thread stores 0.95 ms, staged stores 0.77-0.83 ms, window-row operands 0.67-0.69 ms, trimmed epilogue 0.637 ms.
-// What bounds it now (profiles/r02_stem_rows_ncu.txt): the EPI warps' own latency chain -- TMEM-load data and
-// fixed-latency dependencies at two EPI warps per scheduler; they never wait for the tensor core.  Tried and slower:
-// 16 EPI warps of 16 channels (with and without a setmaxnreg register split), two BUILD groups, a software-pipelined
-// epilogue over 8-channel groups (0.691 ms), spinning instead of suspended mbarrier waits (no change).
+// TMA box stores (tools/time_stem.py, profiles/r03_stem_tma_store.txt; B200 at 1 000 W, alternating with the staged
+// store in one process): 0.636-0.642 -> 0.539-0.542 ms (fp32 output), 0.631 -> 0.531 ms (bf16), bit-identical; the
+// staged store's transposed shared-memory reads, 64-bit address arithmetic and predicated STG.E.128 are gone from the
+// EPI chain.
+// What bounds it (profiles/r02_stem_rows_ncu.txt, before the TMA store): the EPI warps' own latency chain -- TMEM-load
+// data and fixed-latency dependencies at two EPI warps per scheduler; they never wait for the tensor core.  Tried and
+// slower: 16 EPI warps of 16 channels (with and without a setmaxnreg register split), two BUILD groups, a
+// software-pipelined epilogue over 8-channel groups (0.691 ms), spinning instead of suspended mbarrier waits (no change).
+// Tried and not merged: rolling TMEM loads (row g+1's tcgen05.ld issued into each window's registers as soon as row g's
+// maxima have consumed them, and the next tile's first row issued before this tile's store).  A row's three windows
+// and the running maxima are 96 + 32 = 128 registers, so a load in flight before a row is fully folded needs registers
+// 13 warps do not have: every arrangement spilled (188-748 B of spill stores per thread, -Xptxas -v) and ran 1.19-1.82 ms,
+// and a 16-warp setmaxnreg split (EPI 144-160 registers) still spilled 56-360 B in the EPI code.
+#include <cuda.h>
 #include <cuda_bf16.h>
 #include <stdlib.h>
 
@@ -52,8 +64,9 @@ constexpr uint32_t kWinBytes = 4u * kPix1 * 16u;      // one window ROW's P_g: [
 constexpr uint32_t kTileBytes = 3u * kWinBytes;       // three window rows: 24 KB
 constexpr uint32_t kAccCols = 3u * kCh1;              // one window row: three accumulators side by side = UMMA N
 constexpr uint32_t kWBytes = 4u * kAccCols * 16u;     // Wf: [4 chunks][192 rows][16 B] = 12 KB
-constexpr int kStagePitch = 36;                       // floats per staged pixel row (32 channels + 4: conflict-free)
-constexpr uint32_t kStageBytes = 32u * kStagePitch * 4u;  // per EPI warp
+constexpr uint32_t kBoxBytes = 32u * 32u * 4u;        // one EPI warp's output box: 32 pixels x 32 channels (fp32)
+constexpr uint32_t kStageOff = kNBuf1 * kTileBytes + kWBytes;  // two boxes per EPI warp from here (1024-aligned)
+constexpr size_t kSmem1 = kStageOff + 8u * 2u * kBoxBytes + 1024u;  // + the base's alignment to 1024 B
 constexpr uint32_t kTmemCols1 = 512;
 
 struct Conv1TcParams {
@@ -61,21 +74,31 @@ struct Conv1TcParams {
   float shift[kCh1];
 };
 
+__device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
+  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
+}
+__device__ __forceinline__ uint32_t bf162_bits(__nv_bfloat162 p) { return *reinterpret_cast<const uint32_t*>(&p); }
+
 enum { kAFull = 0, kAEmpty = kNBuf1, kAccFull = 2 * kNBuf1, kAccEmpty = 2 * kNBuf1 + 2, kBars1 = 2 * kNBuf1 + 4 };
 
 // OBF16: the channels-last output is written as bf16 (the input of the bf16 blocks of csrc/conv3_tc.cu) instead of fp32
 template <bool LEAKY, bool OBF16>
 __global__ void __launch_bounds__(kThreads1, 1)
 conv1_tc_kernel(const float* __restrict__ x, int64_t total_pix, int H, int Wd, int PH, int PW, float slope,
-                void* __restrict__ out_, const __grid_constant__ Conv1TcParams prm) {
-  extern __shared__ __align__(128) uint8_t s_buf[];  // [kNBuf1][kTileBytes] patches | [kWBytes] weights | [8][kStageBytes] output staging
+                const __grid_constant__ CUtensorMap out_map,
+                const __grid_constant__ Conv1TcParams prm) {
+  // [kNBuf1][kTileBytes] patches | [kWBytes] weights | [8 EPI warps][2][kBoxBytes] output staging, from a 1024-byte
+  // aligned base (the staging boxes are read by TMA with a 128-byte swizzle)
+  extern __shared__ __align__(1024) uint8_t s_raw[];
   __shared__ __align__(8) uint64_t s_bars[kBars1];
   __shared__ uint32_t s_tmem;
   __shared__ __align__(16) float s_shift[kCh1];
 
   const int tid = threadIdx.x;
   const int warp = tid >> 5, lane = tid & 31;
+  uint8_t* s_buf = s_raw + ((1024u - (smem_u32(s_raw) & 1023u)) & 1023u);
   const uint32_t a_base = smem_u32(s_buf);
+  const uint32_t stage_base = a_base + kStageOff;
   const uint32_t w_base = a_base + kNBuf1 * kTileBytes;
   if (tid < kCh1) s_shift[tid] = prm.shift[tid];
   const uint32_t bars = smem_u32(s_bars);
@@ -123,16 +146,10 @@ conv1_tc_kernel(const float* __restrict__ x, int64_t total_pix, int H, int Wd, i
       const int64_t tile = blockIdx.x + it * gridDim.x;
       int64_t pix = tile * kPix1 + tid;
       if (pix >= total_pix) pix = total_pix - 1;  // tail rows recompute the last pixel; never stored
-      int64_t n;
-      uint32_t r;
-      if (total_pix <= 0x7fffffffLL) {  // the usual case: 32-bit division
-        const uint32_t n32 = static_cast<uint32_t>(pix) / per;
-        n = n32;
-        r = static_cast<uint32_t>(pix) - n32 * per;
-      } else {
-        n = pix / per;
-        r = static_cast<uint32_t>(pix - n * per);
-      }
+      // 32-bit division: the host caps total_pix at 2^31 - 1 (TMA coordinates)
+      const uint32_t n32 = static_cast<uint32_t>(pix) / per;
+      const int64_t n = n32;
+      const uint32_t r = static_cast<uint32_t>(pix) - n32 * per;
       const uint32_t ph = r / static_cast<uint32_t>(PW), pw = r - ph * static_cast<uint32_t>(PW);
       const int y0 = 3 * static_cast<int>(ph) - 1, x0 = 3 * static_cast<int>(pw) - 1;
       // validity of the five rows / columns as bit masks: only the first and the last can fall outside (H, Wd >= 3)
@@ -199,7 +216,6 @@ conv1_tc_kernel(const float* __restrict__ x, int64_t total_pix, int H, int Wd, i
     const int e = warp - 4;
     const int half = e >> 2;  // channels 32 half .. 32 half + 31; TMEM lane quadrant = warp & 3 = e & 3
     const uint32_t t_row = tmem_base + (static_cast<uint32_t>((warp & 3) * 32) << 16) + 32u * half;
-    float* stage = reinterpret_cast<float*>(s_buf + kNBuf1 * kTileBytes + kWBytes + static_cast<uint32_t>(e) * kStageBytes);
     uint32_t r = 0;
     for (int64_t it = 0; it < my_tiles; ++it) {
       float best[32];
@@ -227,47 +243,45 @@ conv1_tc_kernel(const float* __restrict__ x, int64_t total_pix, int H, int Wd, i
           }
         }
       }
-      __syncwarp();  // the previous tile's staging reads are done
+      const int64_t tile = blockIdx.x + it * gridDim.x;
+      // + folded shift, activation, and this thread's pixel row into the warp's staging box (16-byte chunks at their
+      // swizzled positions; conflict-free: 8 consecutive lanes hit 8 different chunk columns); one lane stores the box
+      const uint32_t box = stage_base + static_cast<uint32_t>(2 * e + (it & 1)) * kBoxBytes;
+      if (lane == 0) bulk_wait_read<1>();  // the store issued from this box two tiles ago has read it
+      __syncwarp();
 #pragma unroll
       for (int c4 = 0; c4 < 8; ++c4) {
         // one 128-bit broadcast load of four shifts (a scalar load per channel was 12 % of the kernel's stall samples)
         const float4 sh4 = *reinterpret_cast<const float4*>(s_shift + 32 * half + 4 * c4);
         const float sh[4] = {sh4.x, sh4.y, sh4.z, sh4.w};
-        float q[4];
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
-          const float v = best[4 * c4 + k] + sh[k];
-          q[k] = LEAKY ? fmaxf(v, v * slope) : fmaxf(v, 0.f);  // 0 <= slope < 1: max(v, slope v) is LeakyReLU
+          const float x = best[4 * c4 + k] + sh[k];
+          best[4 * c4 + k] = LEAKY ? fmaxf(x, x * slope) : fmaxf(x, 0.f);  // 0 <= slope < 1: max(x, slope x)
         }
-        *reinterpret_cast<float4*>(stage + lane * kStagePitch + 4 * c4) = make_float4(q[0], q[1], q[2], q[3]);
+        if (OBF16) {
+          if (c4 & 1) {  // 8 channels = one 16-byte chunk of the 64-byte row (SWIZZLE_64B: chunk ^= row bits 1-2)
+            const float* q = best + 4 * (c4 - 1);
+            const __nv_bfloat162 p0 = __floats2bfloat162_rn(q[0], q[1]), p1 = __floats2bfloat162_rn(q[2], q[3]);
+            const __nv_bfloat162 p2 = __floats2bfloat162_rn(q[4], q[5]), p3 = __floats2bfloat162_rn(q[6], q[7]);
+            const uint32_t c = static_cast<uint32_t>(c4 >> 1) ^ ((static_cast<uint32_t>(lane) >> 1) & 3u);
+            st_shared_v4(box + 64u * lane + 16u * c, bf162_bits(p0), bf162_bits(p1), bf162_bits(p2), bf162_bits(p3));
+          }
+        } else {  // 4 channels = one 16-byte chunk of the 128-byte row (SWIZZLE_128B: chunk ^= row bits 0-2)
+          const uint32_t c = static_cast<uint32_t>(c4) ^ (static_cast<uint32_t>(lane) & 7u);
+          st_shared_v4(box + 128u * lane + 16u * c, __float_as_uint(best[4 * c4]), __float_as_uint(best[4 * c4 + 1]),
+                       __float_as_uint(best[4 * c4 + 2]), __float_as_uint(best[4 * c4 + 3]));
+        }
       }
+      fence_async_smem();
       __syncwarp();
-      const int64_t tile = blockIdx.x + it * gridDim.x;
-      const int64_t pix0 = tile * kPix1 + (warp & 3) * 32;  // first pixel of this warp's 32
-      if (OBF16) {
-        __nv_bfloat16* out = static_cast<__nv_bfloat16*>(out_);
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const int q = 8 * i + (lane >> 2), c = lane & 3;  // pixel of the warp, 16-byte chunk of its 64-byte half-row
-          const float4 a = *reinterpret_cast<const float4*>(stage + q * kStagePitch + 8 * c);
-          const float4 b = *reinterpret_cast<const float4*>(stage + q * kStagePitch + 8 * c + 4);
-          const __nv_bfloat162 p0 = __floats2bfloat162_rn(a.x, a.y), p1 = __floats2bfloat162_rn(a.z, a.w);
-          const __nv_bfloat162 p2 = __floats2bfloat162_rn(b.x, b.y), p3 = __floats2bfloat162_rn(b.z, b.w);
-          uint4 v;
-          v.x = *reinterpret_cast<const uint32_t*>(&p0); v.y = *reinterpret_cast<const uint32_t*>(&p1);
-          v.z = *reinterpret_cast<const uint32_t*>(&p2); v.w = *reinterpret_cast<const uint32_t*>(&p3);
-          if (pix0 + q < total_pix) *reinterpret_cast<uint4*>(out + (pix0 + q) * kCh1 + 32 * half + 8 * c) = v;
-        }
-      } else {
-        float* out = static_cast<float*>(out_);
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int q = 4 * i + (lane >> 3), c = lane & 7;  // pixel of the warp, 16-byte chunk of its 128-byte half-row
-          const float4 v = *reinterpret_cast<const float4*>(stage + q * kStagePitch + 4 * c);
-          if (pix0 + q < total_pix) *reinterpret_cast<float4*>(out + (pix0 + q) * kCh1 + 32 * half + 4 * c) = v;
-        }
+      if (lane == 0) {  // pixels past total_pix fall outside the tensor map and are not written
+        const int64_t pix0 = tile * kPix1 + (warp & 3) * 32;
+        if (pix0 < total_pix) tma_store_2d(&out_map, box, 32 * half, static_cast<int>(pix0));
+        bulk_commit();
       }
     }
+    if (lane == 0) bulk_wait<0>();  // the output is written and the staging boxes are no longer read
   }
 #undef BAR1
 
@@ -282,12 +296,28 @@ conv1_tc_kernel(const float* __restrict__ x, int64_t total_pix, int H, int Wd, i
 namespace afs {
 namespace {
 
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+EncodeTiledFn encode_tiled_c1() {
+  static EncodeTiledFn fn = nullptr;
+  if (fn == nullptr) {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
+        q == cudaDriverEntryPointSuccess)
+      fn = reinterpret_cast<EncodeTiledFn>(p);
+  }
+  return fn;
+}
+
 template <bool LEAKY, bool OBF16>
-int launch_conv1_tc(const float* x, int64_t total, int H, int Wd, int PH, int PW, float slope, void* out,
-                    const Conv1TcParams& prm, unsigned blocks, size_t smem, cudaStream_t stream) {
+int launch_conv1_tc(const float* x, int64_t total, int H, int Wd, int PH, int PW, float slope, const CUtensorMap& map,
+                    const Conv1TcParams& prm, unsigned blocks, cudaStream_t stream) {
   AFS_CUDA_TRY(cudaFuncSetAttribute(conv1_tc_kernel<LEAKY, OBF16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    static_cast<int>(smem)));
-  conv1_tc_kernel<LEAKY, OBF16><<<blocks, kThreads1, smem, stream>>>(x, total, H, Wd, PH, PW, slope, out, prm);
+                                    static_cast<int>(kSmem1)));
+  conv1_tc_kernel<LEAKY, OBF16><<<blocks, kThreads1, kSmem1, stream>>>(x, total, H, Wd, PH, PW, slope, map, prm);
   AFS_LAUNCH_CHECK();
   return AFS_OK;
 }
@@ -298,23 +328,36 @@ int conv1_tc_fwd(const float* x, int32_t N, int32_t H, int32_t Wd, const float* 
       Wd < 3 || negative_slope < 0.f)
     return AFS_ERR_INVALID_ARG;
   if (C != kCh1) return AFS_ERR_UNSUPPORTED;
-  if ((reinterpret_cast<uintptr_t>(out) & 15) != 0) return AFS_ERR_INVALID_ARG;
+  if ((reinterpret_cast<uintptr_t>(out) & 15) != 0) return AFS_ERR_INVALID_ARG;  // TMA stores need 16-byte alignment
   if (negative_slope >= 1.f) return AFS_ERR_UNSUPPORTED;  // the activation is max(v, slope v)
   if (N == 0) return AFS_OK;
   const int PH = H / 3, PW = Wd / 3;
   const int64_t total = static_cast<int64_t>(N) * PH * PW;
+  if (total > 0x7fffffffLL) return AFS_ERR_UNSUPPORTED;  // TMA coordinates are 32-bit signed
   const int64_t n_tiles = (total + kPix1 - 1) / kPix1;
   Conv1TcParams prm;
   for (int i = 0; i < kCh1 * 9; ++i) prm.w[i] = w_folded_host[i];
   for (int i = 0; i < kCh1; ++i) prm.shift[i] = shift_host[i];
+  // the NHWC output as a [total pixels][64 channels] tensor; one box is one EPI warp's 32 pixels x 32 channels, rows
+  // of 128 B (fp32) or 64 B (bf16) swizzled at their own width
+  EncodeTiledFn fn = encode_tiled_c1();
+  if (fn == nullptr) return AFS_ERR_CUDA;
+  CUtensorMap map;
+  const cuuint64_t gdim[2] = {static_cast<cuuint64_t>(kCh1), static_cast<cuuint64_t>(total)};
+  const cuuint64_t gstride[1] = {static_cast<cuuint64_t>(kCh1) * (out_bf16 ? 2u : 4u)};
+  const cuuint32_t box[2] = {32, 32};
+  const cuuint32_t estr[2] = {1, 1};
+  if (fn(&map, out_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, out, gdim, gstride,
+         box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, out_bf16 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
+         CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+    return AFS_ERR_CUDA;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  const size_t smem = kNBuf1 * kTileBytes + kWBytes + 8 * kStageBytes;
   const unsigned blocks = static_cast<unsigned>(n_tiles < kNumSMs ? n_tiles : kNumSMs);  // persistent: one CTA per SM
   const bool leaky = negative_slope > 0.f;
-  if (leaky && out_bf16) return launch_conv1_tc<true, true>(x, total, H, Wd, PH, PW, negative_slope, out, prm, blocks, smem, stream);
-  if (leaky) return launch_conv1_tc<true, false>(x, total, H, Wd, PH, PW, negative_slope, out, prm, blocks, smem, stream);
-  if (out_bf16) return launch_conv1_tc<false, true>(x, total, H, Wd, PH, PW, negative_slope, out, prm, blocks, smem, stream);
-  return launch_conv1_tc<false, false>(x, total, H, Wd, PH, PW, negative_slope, out, prm, blocks, smem, stream);
+  if (leaky && out_bf16) return launch_conv1_tc<true, true>(x, total, H, Wd, PH, PW, negative_slope, map, prm, blocks, stream);
+  if (leaky) return launch_conv1_tc<true, false>(x, total, H, Wd, PH, PW, negative_slope, map, prm, blocks, stream);
+  if (out_bf16) return launch_conv1_tc<false, true>(x, total, H, Wd, PH, PW, negative_slope, map, prm, blocks, stream);
+  return launch_conv1_tc<false, false>(x, total, H, Wd, PH, PW, negative_slope, map, prm, blocks, stream);
 }
 
 }  // namespace

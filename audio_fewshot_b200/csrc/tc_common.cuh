@@ -157,6 +157,27 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const TensorMap* map, 
       : "memory");
 }
 
+// ---- TMA (tiled 2-D store from shared memory into a bulk async-group).  Groups belong to the issuing thread: the
+// same thread commits them and waits on them.  The writers of the shared-memory box run fence_async_smem() before the
+// store is issued.  Rows and columns outside the tensor map's extent are not written.
+template <typename TensorMap>
+__device__ __forceinline__ void tma_store_2d(const TensorMap* map, uint32_t src, int c0, int c1) {
+  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%1, %2}], [%3];" ::"l"(map), "r"(c0),
+               "r"(c1), "r"(src)
+               : "memory");
+}
+__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+// at most N of this thread's groups still read shared memory (their boxes before that may be rewritten)
+template <int N>
+__device__ __forceinline__ void bulk_wait_read() {
+  asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
+}
+// at most N of this thread's groups are incomplete (their global writes included)
+template <int N>
+__device__ __forceinline__ void bulk_wait() {
+  asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory");
+}
+
 // ---- cp.async (16-byte, L2 only; src_bytes < 16 zero-fills the rest)
 __device__ __forceinline__ void cp_async16(uint32_t dst, const void* src, uint32_t src_bytes) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
