@@ -38,22 +38,6 @@ constexpr int kBThreads = 448;
 constexpr int kBAcc = 4;                      // accumulators: two per epilogue group
 constexpr int kAStride = kBC + 1;
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_tiled_b() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn == nullptr) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
-
 struct BBars {
   uint64_t full[kBStages], lo_ready[kBStages], empty[kBStages], acc_full[kBAcc], acc_empty[kBAcc];
 };
@@ -276,7 +260,7 @@ bdc_tc_kernel(const __grid_constant__ CUtensorMap map_x, int B, int n_chunks, co
 int bdc_fwd_tc(const float* x, int32_t B, int32_t C, int32_t M, const float* log_temp, int32_t triu, float* out,
                cudaStream_t stream) {
   if (C != kBC || M % 4 != 0 || (reinterpret_cast<uintptr_t>(x) & 15) != 0) return AFS_ERR_UNSUPPORTED;
-  EncodeTiledFn fn = encode_tiled_b();
+  EncodeTiledFn fn = encode_tiled();
   if (fn == nullptr) return AFS_ERR_UNSUPPORTED;
   CUtensorMap map;
   const cuuint64_t gdim[2] = {static_cast<cuuint64_t>(M), static_cast<cuuint64_t>(B) * kBC};

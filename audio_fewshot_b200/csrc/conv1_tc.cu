@@ -296,22 +296,6 @@ conv1_tc_kernel(const float* __restrict__ x, int64_t total_pix, int H, int Wd, i
 namespace afs {
 namespace {
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_tiled_c1() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn == nullptr) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
-
 template <bool LEAKY, bool OBF16>
 int launch_conv1_tc(const float* x, int64_t total, int H, int Wd, int PH, int PW, float slope, const CUtensorMap& map,
                     const Conv1TcParams& prm, unsigned blocks, cudaStream_t stream) {
@@ -340,7 +324,7 @@ int conv1_tc_fwd(const float* x, int32_t N, int32_t H, int32_t Wd, const float* 
   for (int i = 0; i < kCh1; ++i) prm.shift[i] = shift_host[i];
   // the NHWC output as a [total pixels][64 channels] tensor; one box is one EPI warp's 32 pixels x 32 channels, rows
   // of 128 B (fp32) or 64 B (bf16) swizzled at their own width
-  EncodeTiledFn fn = encode_tiled_c1();
+  tc::EncodeTiledFn fn = tc::encode_tiled();
   if (fn == nullptr) return AFS_ERR_CUDA;
   CUtensorMap map;
   const cuuint64_t gdim[2] = {static_cast<cuuint64_t>(kCh1), static_cast<cuuint64_t>(total)};

@@ -48,22 +48,6 @@ constexpr int kCols2 = 128;   // UMMA N
 constexpr int kMaxWay2 = 32;
 constexpr uint32_t kAtomBytes = 128u * 128u;  // one [128 rows x 32 floats] swizzle-128B operand block
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_tiled() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn == nullptr) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
-
 // [rows, C] fp32 row-major tensor, boxes of 32 channels x 128 rows, 128B swizzle, zero fill out of bounds
 bool make_map(CUtensorMap* map, const float* base, uint64_t rows, uint32_t C) {
   EncodeTiledFn fn = encode_tiled();

@@ -30,25 +30,9 @@ constexpr int kPRows = 128, kPCols = 32, kPStages = 6;
 constexpr uint32_t kABytes = kPRows * 128u, kBBytes = kPCols * 128u, kStageBytesP = kABytes + kBBytes;
 constexpr int kPThreads = 192;
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_tiled_p() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn == nullptr) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
-
 // [rows, D] fp32 (row stride ld floats), boxes of 32 features x box_rows rows, 128B swizzle, zero fill out of bounds
 bool make_map_p(CUtensorMap* map, const float* base, uint64_t rows, uint32_t D, uint64_t ld, uint32_t box_rows) {
-  EncodeTiledFn fn = encode_tiled_p();
+  EncodeTiledFn fn = encode_tiled();
   if (fn == nullptr) return false;
   const cuuint64_t gdim[2] = {D, rows};
   const cuuint64_t gstride[1] = {ld * sizeof(float)};

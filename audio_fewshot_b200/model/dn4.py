@@ -20,8 +20,7 @@ class DN4(MetricModel):
         image, repeats, support_size = self._unpack(batch)
         feat = self.emb_func(image)  # [N, C, H, W]
         tab = self._table(feat.shape[0], repeats, support_size)
-        c = feat.shape[1]
-        precision = self.precision if (c % 32 == 0 or (c % 8 == 0 and c <= 128)) else "fp32"
+        precision = self.precision if ops.dn4_tc_supported(feat.shape[1]) else "fp32"
         output, _, _ = ops.dn4_scores(feat, tab.cls_row, tab.E, tab.W, tab.S, self.n_k, precision=precision)
         _, acc, _ = ops.vote_acc(output, tab.q_start, tab.q_target)
         return output, acc

@@ -485,6 +485,12 @@ def proto_logits(feat, cls_row, E, W, S, mode="euclidean", want_pred=False, prec
     return (logits, pred) if want_pred else logits
 
 
+def dn4_tc_supported(C):
+    """Channel counts the tensor-core DN4 head (precision="tf32") is built for: multiples of 32 up to 4096
+    (csrc/dn4_tc2.cu) and multiples of 8 up to 128 (csrc/dn4_tc.cu).  Other maps run the fp32 head."""
+    return C % 8 == 0 and (C <= 128 or (C % 32 == 0 and C <= 4096))
+
+
 def _dn4_tc_call(feat, cls_row, E, W, S, n_k, want_topk, want_pred, staged=False):
     """Tensor-core (tcgen05 TF32) DN4 head; same outputs as _dn4_call.  C % 32 == 0 runs the TMA-fed
     pipeline (csrc/dn4_tc2.cu); other C % 8 == 0 widths (or staged=True) the register-staged kernel
@@ -558,8 +564,7 @@ def dn4_scores(feat, cls_row, E, W, S, n_k, want_topk=False, want_pred=False, pr
     """DN4 head.  feat [N, C, H, W] (or [N, C, HW]) -> score [NQ, W] (+ topk_idx [NQ, W, HW, n_k], pred).
     Differentiable w.r.t. feat when it requires grad (top-k selection held fixed, as torch.topk's backward).
     precision: "fp32" = bit-stable SIMT path (parity with the reference's indices); "tf32" = tcgen05 tensor-core
-    path (C % 32 == 0 up to 4096 channels, or C % 8 == 0 up to 128), scores to ~1e-4, indices may differ at
-    near-ties."""
+    path (the widths dn4_tc_supported accepts), scores to ~1e-4, indices may differ at near-ties."""
     if precision not in ("fp32", "tf32", "tf32_staged"):
         raise ValueError("precision must be 'fp32', 'tf32' or 'tf32_staged'")
     if torch.is_grad_enabled() and isinstance(feat, torch.Tensor) and feat.requires_grad:

@@ -315,7 +315,7 @@ int afs_dn4_fwd_tc(const float* feat, const int32_t* cls_row, int32_t N, int32_t
 /* (2b'') Warp-specialised version of (2b'): a pre-pass writes normalised TF32 descriptors K-major, the main
  * kernel feeds tcgen05.mma from TMA (cp.async.bulk.tensor, 128B swizzle) through a two-stage mbarrier
  * pipeline with two TMEM accumulators, so loads, MMAs and the top-k epilogue overlap.  C % 32 == 0 and
- * C <= 128 (AFS_ERR_UNSUPPORTED otherwise); ws (256-byte aligned): afs_dn4_tc2_workspace_bytes().      */
+ * C <= 4096 (AFS_ERR_UNSUPPORTED otherwise); ws (256-byte aligned): afs_dn4_tc2_workspace_bytes().     */
 size_t afs_dn4_tc2_workspace_bytes(int32_t N, int32_t E, int32_t W, int32_t S, int32_t C, int32_t HW);
 int afs_dn4_fwd_tc2(const float* feat, const int32_t* cls_row, int32_t N, int32_t E, int32_t W, int32_t S,
                     int32_t C, int32_t HW, int32_t n_k, float* score, int32_t* topk_idx, int32_t* pred,

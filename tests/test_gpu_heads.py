@@ -238,14 +238,16 @@ def test_dn4_tensor_core_path_ragged_multi_tile_and_unsupported(cuda):
     from audio_fewshot_b200 import ops
     from audio_fewshot_b200._lib import AfsError
     rng = np.random.default_rng(15)
-    E, W, S, Q, C, H, Wd, n_k = 3, 5, 8, 3, 64, 4, 5, 3  # S*HW = 160 support descriptors: two column tiles
-    rep = rng.integers(1, 4, size=E * W * Q)
-    n = E * W * S + int(rep.sum())
-    feat = torch.from_numpy(np.abs(rng.standard_normal((n, C, H, Wd))).astype(np.float32)).to(cuda)
-    tab = ragged_table(E, W, S, Q, rep, cuda)
-    a, _, _ = ops.dn4_scores(feat, tab.cls_row, E, W, S, n_k)
-    b, _, _ = ops.dn4_scores(feat, tab.cls_row, E, W, S, n_k, precision="tf32")
-    assert (a - b).abs().max().item() <= 3e-4 * a.abs().max().item()
+    for C in (64, 8, 40, 72, 120):  # every width dn4_tc_supported admits below 128 channels has a tensor-core kernel
+        assert ops.dn4_tc_supported(C)
+        E, W, S, Q, H, Wd, n_k = 3, 5, 8, 3, 4, 5, 3  # S*HW = 160 support descriptors: two column tiles
+        rep = rng.integers(1, 4, size=E * W * Q)
+        n = E * W * S + int(rep.sum())
+        feat = torch.from_numpy(np.abs(rng.standard_normal((n, C, H, Wd))).astype(np.float32)).to(cuda)
+        tab = ragged_table(E, W, S, Q, rep, cuda)
+        a, _, _ = ops.dn4_scores(feat, tab.cls_row, E, W, S, n_k)
+        b, _, _ = ops.dn4_scores(feat, tab.cls_row, E, W, S, n_k, precision="tf32")
+        assert (a - b).abs().max().item() <= 3e-4 * a.abs().max().item(), C
     # C = 640 (ResNet-12 maps): K-streaming schedule, ragged windows, three column tiles with a partial last one
     E, W, S, Q, C, H, Wd = 2, 5, 5, 2, 640, 8, 9
     rep = rng.integers(1, 3, size=E * W * Q)
@@ -256,10 +258,12 @@ def test_dn4_tensor_core_path_ragged_multi_tile_and_unsupported(cuda):
     b, ib, _ = ops.dn4_scores(feat, tab.cls_row, E, W, S, n_k, want_topk=True, precision="tf32")
     assert (a - b).abs().max().item() <= 3e-4 * a.abs().max().item()
     assert (ia != ib).float().mean().item() <= 0.02
-    odd = torch.rand(2 * 5 * 3, 136, 2, 2, device=cuda)  # > 128 channels and not a multiple of 32: no tensor-core kernel
     tab2 = ragged_table(2, 5, 1, 2, np.ones(20, dtype=np.int64), cuda)
-    with pytest.raises(AfsError):
-        ops.dn4_scores(odd, tab2.cls_row, 2, 5, 1, 2, precision="tf32")
+    for C in (36, 136):  # not a multiple of 8, or > 128 channels and not a multiple of 32: no tensor-core kernel
+        assert not ops.dn4_tc_supported(C)
+        odd = torch.rand(2 * 5 * 3, C, 2, 2, device=cuda)
+        with pytest.raises(AfsError):
+            ops.dn4_scores(odd, tab2.cls_row, 2, 5, 1, 2, precision="tf32")
 
 
 def test_dn4_ragged_matches_oracle(cuda):
