@@ -56,7 +56,6 @@ SIGNATURES = {
     "afs_logmel_plan_create": (C.c_int, [C.POINTER(LogMelCfg), C.c_void_p, C.c_void_p, C.c_int,
                                          C.POINTER(C.c_void_p)]),
     "afs_logmel_plan_destroy": (C.c_int, [C.c_void_p]),
-    "afs_logmel_plan_set_engine": (C.c_int, [C.c_void_p, C.c_int32]),
     "afs_logmel_num_frames": (C.c_int, [C.c_void_p, C.c_int64]),
     "afs_logmel_fwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p,
                                  C.POINTER(AugCfg), C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p]),

@@ -1,7 +1,8 @@
-// Fused waveform -> normalised log-mel front-end for sm_100a.
+// Fused waveform -> normalised log-mel front-end for sm_100a: the plan, the C ABI entry points, and the radix-8
+// engine, which serves augmented launches (plain launches run the pair engine of logmel_pair.cu).
 //
-// One launch does: (optional Philox gain / time-shift / additive-noise
-// augmentation) -> reflect padding -> framing -> window -> 1024-point real FFT
+// One launch does: Philox gain / time-shift / additive-noise
+// augmentation -> reflect padding -> framing -> window -> 1024-point real FFT
 // (512-point complex radix-8 x3 in registers + shared-memory exchanges) ->
 // power -> banded mel projection -> log_mult*log10(. + eps) -> (. - mean)/std
 // -> [B, 1, n_mels, T].  Spectra never leave the SM; HBM sees the waveform once
@@ -56,38 +57,27 @@ __device__ __forceinline__ void group_bar(int grp) {
 // starts at sample s0.  Issued one frame ahead of their use so the global-load latency hides behind the
 // previous frame's FFT.
 // R0 = 0 loads the whole frame, R0 = 4 only its second half (see the hop == n_fft/2 reuse in the kernel).
-template <bool AUG, typename S, int R0>
+template <typename S, int R0>
 __device__ __forceinline__ void load_frame(const S* __restrict__ x, int64_t s0, int64_t L, int t,
                                            const AugState& aug, float2 (&raw)[8]) {
   const bool interior = (s0 >= 0) && (s0 + kNfft <= L);
-  if (!AUG && interior && ((reinterpret_cast<uintptr_t>(x + s0) & (2 * sizeof(S) - 1)) == 0)) {
-    const S* xb = x + s0 + 2 * t;
 #pragma unroll
-    for (int r = R0; r < 8; ++r) raw[r] = ld_pair(xb + 128 * r, aug.pcm_scale);
-  } else {
-#pragma unroll
-    for (int r = R0; r < 8; ++r) {
-      int64_t i0 = s0 + 2 * (t + 64 * r), i1 = i0 + 1;
-      if (!interior) {
-        i0 = reflect_index(i0, L);
-        i1 = reflect_index(i1, L);
-      }
-      if (AUG) {
-        if (interior && (i0 & 1) == 0) {
-          raw[r] = aug_pair(x, i0, L, aug);
-        } else {
-          raw[r].x = aug_sample(x, i0, L, aug);
-          raw[r].y = aug_sample(x, i1, L, aug);
-        }
-      } else {
-        raw[r].x = ld_sample(x + i0, aug.pcm_scale);
-        raw[r].y = ld_sample(x + i1, aug.pcm_scale);
-      }
+  for (int r = R0; r < 8; ++r) {
+    int64_t i0 = s0 + 2 * (t + 64 * r), i1 = i0 + 1;
+    if (!interior) {
+      i0 = reflect_index(i0, L);
+      i1 = reflect_index(i1, L);
+    }
+    if (interior && (i0 & 1) == 0) {
+      raw[r] = aug_pair(x, i0, L, aug);
+    } else {
+      raw[r].x = aug_sample(x, i0, L, aug);
+      raw[r].y = aug_sample(x, i1, L, aug);
     }
   }
 }
 
-template <bool AUG, typename S>
+template <typename S>
 __global__ void __launch_bounds__(kThreads, 2) logmel_kernel(const Params p) {
   extern __shared__ __align__(16) float smem[];
   float* s_w = smem;
@@ -142,7 +132,7 @@ __global__ void __launch_bounds__(kThreads, 2) logmel_kernel(const Params p) {
 
     AugState aug;
     aug.pcm_scale = p.pcm_scale;
-    if (AUG) init_clip_aug(aug, p, clip);
+    init_clip_aug(aug, p, clip);
 
     const int t0 = chunk * kFramesPerCta;
     const int nfr = min(kFramesPerCta, p.T - t0);
@@ -150,47 +140,20 @@ __global__ void __launch_bounds__(kThreads, 2) logmel_kernel(const Params p) {
     const int f_end = min(f_begin + kFramesPerGroup, nfr);
 
     float2 raw[8];
-    if (f_begin < f_end) load_frame<AUG, S, 0>(x, static_cast<int64_t>(t0 + f_begin) * p.hop - p.pad, p.L, t, aug, raw);
-    // When every frame of this group lies inside the clip and starts on an aligned sample pair, the prefetch is
-    // four 64-bit loads off a pointer that advances by hop -- the general path spends ~35 instructions per frame on
-    // 64-bit index arithmetic and the interior / alignment / reflect selection.
-    bool lean = false;
-    const S* fptr = x;
-    if constexpr (!AUG) {
-      if (f_begin < f_end) {
-        const int64_t s_first = static_cast<int64_t>(t0 + f_begin) * p.hop - p.pad;
-        const int64_t s_last = static_cast<int64_t>(t0 + f_end - 1) * p.hop - p.pad;
-        lean = (p.hop & 1) == 0 && s_first >= 0 && s_last + kNfft <= p.L &&
-               (reinterpret_cast<uintptr_t>(x + s_first) & (2 * sizeof(S) - 1)) == 0;
-        fptr = x + s_first + 2 * t;
-      }
-    }
+    if (f_begin < f_end) load_frame<S, 0>(x, static_cast<int64_t>(t0 + f_begin) * p.hop - p.pad, p.L, t, aug, raw);
 
     for (int fl = f_begin; fl < f_end; ++fl) {
       float2 zp[8];  // complex numbers as (re, im) register pairs, 64-bit exchanges (logmel_fft.cuh)
 #pragma unroll
       for (int r = 0; r < 8; ++r) zp[r] = p_mul(raw[r], win[r]);
-      if (!AUG && lean) {
-        if (fl + 1 < f_end) {
-          fptr += p.hop;  // sample 2 (t + 64 r) of the next frame is fptr[128 r]
-          if (half_overlap) {
-#pragma unroll
-            for (int r = 0; r < 4; ++r) raw[r] = raw[r + 4];
-#pragma unroll
-            for (int r = 4; r < 8; ++r) raw[r] = ld_pair(fptr + 128 * r, aug.pcm_scale);
-          } else {
-#pragma unroll
-            for (int r = 0; r < 8; ++r) raw[r] = ld_pair(fptr + 128 * r, aug.pcm_scale);
-          }
-        }
-      } else if (fl + 1 < f_end) {  // prefetch the next frame while this one is transformed
+      if (fl + 1 < f_end) {  // prefetch the next frame while this one is transformed
         const int64_t s_next = static_cast<int64_t>(t0 + fl + 1) * p.hop - p.pad;
         if (half_overlap) {  // its first half is this frame's second half: sample index s_next + 2(t+64r) = s0 + 2(t+64(r+4))
 #pragma unroll
           for (int r = 0; r < 4; ++r) raw[r] = raw[r + 4];
-          load_frame<AUG, S, 4>(x, s_next, p.L, t, aug, raw);
+          load_frame<S, 4>(x, s_next, p.L, t, aug, raw);
         } else {
-          load_frame<AUG, S, 0>(x, s_next, p.L, t, aug, raw);
+          load_frame<S, 0>(x, s_next, p.L, t, aug, raw);
         }
       }
       const int slot = (fl - f_begin) % kMelBatch;
@@ -267,7 +230,6 @@ extern "C" int afs_logmel_plan_create(const afs_logmel_cfg* cfg, const float* fb
   plan->nnz = static_cast<int>(weights.size());
   plan->d_window = nullptr; plan->d_tw1024 = nullptr; plan->d_band = nullptr; plan->d_weights = nullptr;
   plan->d_band64 = nullptr; plan->d_weights64 = nullptr;
-  plan->engine = AFS_LOGMEL_ENGINE_AUTO;
 
   int prev = 0;
   cudaError_t e = cudaGetDevice(&prev);
@@ -285,10 +247,8 @@ extern "C" int afs_logmel_plan_create(const afs_logmel_cfg* cfg, const float* fb
   if (e == cudaSuccess) e = cudaMemcpy(plan->d_band64, band64.data(), band64.size() * sizeof(int), cudaMemcpyHostToDevice);
   if (e == cudaSuccess) e = cudaMemcpy(plan->d_weights64, weights64.data(), weights64.size() * sizeof(float), cudaMemcpyHostToDevice);
   const int smem = static_cast<int>(kSmemBytes);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_kernel<false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_kernel<false, int16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_kernel<true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_kernel<true, int16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_kernel<int16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e == cudaSuccess) e = logmel::pair_prepare();
   cudaSetDevice(prev);
   if (e != cudaSuccess) {
@@ -308,14 +268,6 @@ extern "C" int afs_logmel_plan_destroy(afs_logmel_plan* plan) {
   cudaFree(plan->d_band64);
   cudaFree(plan->d_weights64);
   delete plan;
-  return AFS_OK;
-}
-
-extern "C" int afs_logmel_plan_set_engine(afs_logmel_plan* plan, int32_t engine) {
-  if (plan == nullptr ||
-      (engine != AFS_LOGMEL_ENGINE_FFT && engine != AFS_LOGMEL_ENGINE_PAIR && engine != AFS_LOGMEL_ENGINE_AUTO))
-    return AFS_ERR_INVALID_ARG;
-  plan->engine = engine;
   return AFS_OK;
 }
 
@@ -343,33 +295,25 @@ int logmel_launch(const afs_logmel_plan* plan, const S* wav, float pcm_scale, in
   const int T = num_frames(cfg, L);
   if (B == 0 || T <= 0) return AFS_OK;
 
-  Params p;
+  Params p{};
   p.wav = wav; p.pcm_scale = pcm_scale; p.out = out; p.mean = mean; p.stdv = std;
   p.window = plan->d_window; p.tw1024 = plan->d_tw1024; p.band = plan->d_band; p.weights = plan->d_weights;
   p.L = L; p.nnz = plan->nnz; p.B = B; p.T = T; p.hop = cfg.hop; p.n_mels = cfg.n_mels; p.pad = pad;
   p.chunks = (T + kFramesPerCta - 1) / kFramesPerCta;
   p.log_mult = cfg.log_mult; p.log_eps = cfg.log_eps;
-  p.gain_lo = p.gain_hi = p.noise_lo = p.noise_hi = 0.f; p.max_shift = 0;
-  p.seed_lo = static_cast<uint32_t>(seed); p.seed_hi = static_cast<uint32_t>(seed >> 32);
-  p.first_clip = first_clip_index;
   const int64_t items = static_cast<int64_t>(B) * p.chunks;
   if (items > 0x7fffffffLL) return AFS_ERR_UNSUPPORTED;
-  // persistent: 2 resident CTAs per SM (128 registers x 256 threads, 100 KB of shared memory each) walk the items
-  const int64_t grid = items < 2 * kNumSMs ? items : 2 * kNumSMs;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  const unsigned g = static_cast<unsigned>(grid);
-  if (aug != nullptr) {
-    p.gain_lo = aug->gain_db_lo; p.gain_hi = aug->gain_db_hi;
-    p.noise_lo = aug->noise_std_lo; p.noise_hi = aug->noise_std_hi;
-    p.max_shift = aug->max_shift;
-  }
-  if (plan->engine == AFS_LOGMEL_ENGINE_PAIR || (plan->engine == AFS_LOGMEL_ENGINE_AUTO && aug == nullptr))
-    return logmel::pair_launch<S>(plan, p, aug != nullptr, stream);
-  if (aug != nullptr) {
-    logmel_kernel<true, S><<<g, kThreads, kSmemBytes, stream>>>(p);
-  } else {
-    logmel_kernel<false, S><<<g, kThreads, kSmemBytes, stream>>>(p);
-  }
+  if (aug == nullptr) return logmel::pair_launch<S>(plan, p, stream);
+
+  p.gain_lo = aug->gain_db_lo; p.gain_hi = aug->gain_db_hi;
+  p.noise_lo = aug->noise_std_lo; p.noise_hi = aug->noise_std_hi;
+  p.max_shift = aug->max_shift;
+  p.seed_lo = static_cast<uint32_t>(seed); p.seed_hi = static_cast<uint32_t>(seed >> 32);
+  p.first_clip = first_clip_index;
+  // persistent: 2 resident CTAs per SM (128 registers x 256 threads, 100 KB of shared memory each) walk the items
+  const unsigned grid = static_cast<unsigned>(items < 2 * kNumSMs ? items : 2 * kNumSMs);
+  logmel_kernel<S><<<grid, kThreads, kSmemBytes, stream>>>(p);
   AFS_LAUNCH_CHECK();
   return AFS_OK;
 }

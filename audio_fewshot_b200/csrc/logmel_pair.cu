@@ -1,6 +1,7 @@
-// Fused waveform -> normalised log-mel, warp-per-frame-pair engine (AFS_LOGMEL_ENGINE_PAIR) for sm_100a.
+// Fused waveform -> normalised log-mel, warp-per-frame-pair engine for sm_100a: runs every launch without waveform
+// augmentation.
 //
-// Same stage and same contract as logmel.cu (augmentation -> reflect padding -> framing -> window -> 1024-point real
+// Same stage and same contract as logmel.cu (reflect padding -> framing -> window -> 1024-point real
 // DFT -> power -> banded mel projection -> log -> normalise -> [B, 1, n_mels, T]; algorithmic bytes per clip
 // 4 L + 4 n_mels T), different decomposition: a WARP transforms two frames at a time as one 1024-point complex FFT
 // (logmel_pair.cuh) -- one shared-memory exchange per frame PAIR and an in-warp shuffle split instead of three
@@ -21,7 +22,6 @@
 #include "logmel_core.cuh"
 #include "logmel_pair.cuh"
 #include "logmel_plan.cuh"
-#include "philox.cuh"
 
 namespace afs {
 namespace {
@@ -50,24 +50,24 @@ struct RawN {
   static constexpr int boff = HALF ? 16 : 32;
 };
 
-// Interior pair without augmentation: value m of the fetch list straight from memory.
+// Interior pair: value m of the fetch list straight from memory.
 template <typename S, bool HALF>
 __device__ __forceinline__ float ld_fast(const S* xa, int hop, int m, float pcm_scale) {
   if (HALF || m < 32) return ld_sample(xa + 32 * m, pcm_scale);
   return ld_sample(xa + hop + 32 * (m - 32), pcm_scale);
 }
 
-// Raw (augmented, reflect-padded, not yet windowed) samples of the frame pair (fa, fa + 1) of one clip: lane l holds
-// sample l + 32 m of frame a in raw[m] and of frame b in raw[boff + m].  M0 = 16 (HALF only): raw[0..15] were carried
-// over from the previous pair.  The general path: clip edges (reflection), missing second frame, augmentation.
-template <bool AUG, typename S, bool HALF, int M0>
+// Raw (reflect-padded, not yet windowed) samples of the frame pair (fa, fa + 1) of one clip: lane l holds sample
+// l + 32 m of frame a in raw[m] and of frame b in raw[boff + m].  M0 = 16 (HALF only): raw[0..15] were carried over
+// from the previous pair.  The general path: clip edges (reflection), missing second frame.
+template <typename S, bool HALF, int M0>
 __device__ __forceinline__ void load_pair(const S* __restrict__ x, int64_t L, int64_t s0, int hop, bool b_exists, int lane,
-                                          const AugState& aug, float (&raw)[RawN<HALF>::n]) {
+                                          float pcm_scale, float (&raw)[RawN<HALF>::n]) {
   constexpr int n = RawN<HALF>::n;
-  if (!AUG && s0 >= 0 && s0 + (HALF ? 1536 : static_cast<int64_t>(hop) + kNfft) <= L) {  // interior pair
+  if (s0 >= 0 && s0 + (HALF ? 1536 : static_cast<int64_t>(hop) + kNfft) <= L) {  // interior pair
     const S* xa = x + s0 + lane;
 #pragma unroll
-    for (int m = M0; m < n; ++m) raw[m] = ld_fast<S, HALF>(xa, hop, m, aug.pcm_scale);
+    for (int m = M0; m < n; ++m) raw[m] = ld_fast<S, HALF>(xa, hop, m, pcm_scale);
     return;
   }
 #pragma unroll
@@ -77,13 +77,13 @@ __device__ __forceinline__ void load_pair(const S* __restrict__ x, int64_t L, in
     float v = 0.f;
     if (!of_b_only || b_exists) {
       idx = reflect_index(idx, L);
-      v = AUG ? aug_sample(x, idx, L, aug) : ld_sample(x + idx, aug.pcm_scale);
+      v = ld_sample(x + idx, pcm_scale);
     }
     raw[m] = v;
   }
 }
 
-template <bool AUG, typename S, bool HALF>
+template <typename S, bool HALF>
 __global__ void __launch_bounds__(kPThreads, 1) logmel_pair_kernel(const Params p) {
   extern __shared__ __align__(16) float smem[];
   const int nnz_pad = (p.nnz + 3) & ~3;
@@ -132,13 +132,11 @@ __global__ void __launch_bounds__(kPThreads, 1) logmel_pair_kernel(const Params 
   int q = static_cast<int>(g_begin - static_cast<int64_t>(clip) * ppc);
   int col_lo = 2 * (q & 3);  // first tile column this warp owns in its current chunk
 
-  AugState aug;
-  aug.pcm_scale = p.pcm_scale;
+  const float pcm_scale = p.pcm_scale;  // a local: p.pcm_scale at every load spills in the int16 HALF kernel
   float raw[NR];
   {
-    if (AUG) init_clip_aug(aug, p, clip);
     const S* x = static_cast<const S*>(p.wav) + static_cast<int64_t>(clip) * p.L;
-    load_pair<AUG, S, HALF, 0>(x, p.L, static_cast<int64_t>(2 * q) * p.hop - p.pad, p.hop, 2 * q + 1 < p.T, lane, aug, raw);
+    load_pair<S, HALF, 0>(x, p.L, static_cast<int64_t>(2 * q) * p.hop - p.pad, p.hop, 2 * q + 1 < p.T, lane, pcm_scale, raw);
   }
 
   while (left > 0) {
@@ -177,13 +175,12 @@ __global__ void __launch_bounds__(kPThreads, 1) logmel_pair_kernel(const Params 
 #pragma unroll
     for (int k2 = 0; k2 < 16; ++k2) {
       if (k2 == 8 && have_next) {  // z[0..7] and z[24..31] have retired: room for the next pair's samples
-        if (AUG && nclip != clip) init_clip_aug(aug, p, nclip);
         const S* nx = static_cast<const S*>(p.wav) + static_cast<int64_t>(nclip) * p.L;
         const int64_t ns0 = static_cast<int64_t>(2 * nq) * p.hop - p.pad;
         if (carry) {
-          load_pair<AUG, S, HALF, HALF ? 16 : 0>(nx, p.L, ns0, p.hop, 2 * nq + 1 < p.T, lane, aug, raw);
+          load_pair<S, HALF, HALF ? 16 : 0>(nx, p.L, ns0, p.hop, 2 * nq + 1 < p.T, lane, pcm_scale, raw);
         } else {
-          load_pair<AUG, S, HALF, 0>(nx, p.L, ns0, p.hop, 2 * nq + 1 < p.T, lane, aug, raw);
+          load_pair<S, HALF, 0>(nx, p.L, ns0, p.hop, 2 * nq + 1 < p.T, lane, pcm_scale, raw);
         }
       }
       const float2 src = pair_split_src(lane, z, k2);
@@ -243,7 +240,7 @@ __global__ void __launch_bounds__(kPThreads, 1) logmel_pair_kernel(const Params 
 namespace logmel {
 
 template <typename S>
-int pair_launch(const afs_logmel_plan* plan, const Params& p_in, bool aug, cudaStream_t stream) {
+int pair_launch(const afs_logmel_plan* plan, const Params& p_in, cudaStream_t stream) {
   Params p = p_in;
   p.band = plan->d_band64;
   p.weights = plan->d_weights64;
@@ -254,13 +251,8 @@ int pair_launch(const afs_logmel_plan* plan, const Params& p_in, bool aug, cudaS
   const int64_t ctas = (n_pairs + kPWarps - 1) / kPWarps;
   const unsigned grid = static_cast<unsigned>(ctas < kNumSMs ? ctas : kNumSMs);
   const bool half = p.hop * 2 == kNfft;
-  if (aug) {
-    if (half) logmel_pair_kernel<true, S, true><<<grid, kPThreads, smem, stream>>>(p);
-    else logmel_pair_kernel<true, S, false><<<grid, kPThreads, smem, stream>>>(p);
-  } else {
-    if (half) logmel_pair_kernel<false, S, true><<<grid, kPThreads, smem, stream>>>(p);
-    else logmel_pair_kernel<false, S, false><<<grid, kPThreads, smem, stream>>>(p);
-  }
+  if (half) logmel_pair_kernel<S, true><<<grid, kPThreads, smem, stream>>>(p);
+  else logmel_pair_kernel<S, false><<<grid, kPThreads, smem, stream>>>(p);
   AFS_LAUNCH_CHECK();
   return AFS_OK;
 }
@@ -268,10 +260,8 @@ int pair_launch(const afs_logmel_plan* plan, const Params& p_in, bool aug, cudaS
 template <typename S>
 static cudaError_t pair_prepare_t() {
   const int smem = 227 * 1024;
-  cudaError_t e = cudaFuncSetAttribute(logmel_pair_kernel<true, S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_pair_kernel<true, S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_pair_kernel<false, S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_pair_kernel<false, S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  cudaError_t e = cudaFuncSetAttribute(logmel_pair_kernel<S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_pair_kernel<S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   return e;
 }
 
@@ -282,8 +272,8 @@ cudaError_t pair_prepare() {
   return e;
 }
 
-template int pair_launch<float>(const afs_logmel_plan*, const Params&, bool, cudaStream_t);
-template int pair_launch<int16_t>(const afs_logmel_plan*, const Params&, bool, cudaStream_t);
+template int pair_launch<float>(const afs_logmel_plan*, const Params&, cudaStream_t);
+template int pair_launch<int16_t>(const afs_logmel_plan*, const Params&, cudaStream_t);
 
 }  // namespace logmel
 }  // namespace afs

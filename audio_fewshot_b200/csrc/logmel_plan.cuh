@@ -12,7 +12,6 @@ struct afs_logmel_plan {
   afs_logmel_cfg cfg;
   int device;
   int nnz;
-  int engine;        // AFS_LOGMEL_ENGINE_*
   float* d_window;   // [1024]
   float2* d_tw1024;  // [1024]
   int* d_band;       // [3][128]: lo, len, off
@@ -55,11 +54,6 @@ struct AugState {
 __device__ __forceinline__ float ld_sample(const float* p, float) { return __ldg(p); }
 __device__ __forceinline__ float ld_sample(const int16_t* p, float s) {
   return __fmul_rn(static_cast<float>(__ldg(p)), s);
-}
-__device__ __forceinline__ float2 ld_pair(const float* p, float) { return __ldg(reinterpret_cast<const float2*>(p)); }
-__device__ __forceinline__ float2 ld_pair(const int16_t* p, float s) {
-  const short2 v = __ldg(reinterpret_cast<const short2*>(p));
-  return make_float2(__fmul_rn(static_cast<float>(v.x), s), __fmul_rn(static_cast<float>(v.y), s));
 }
 
 // One augmented sample y[idx] = g * x[idx - k] + sigma * n[idx]; n[2i], n[2i+1]
@@ -132,7 +126,7 @@ inline int num_frames(const afs_logmel_cfg& cfg, int64_t L) {
 // logmel_pair.cu
 cudaError_t pair_prepare();
 template <typename S>
-int pair_launch(const afs_logmel_plan* plan, const Params& p, bool aug, cudaStream_t stream);
+int pair_launch(const afs_logmel_plan* plan, const Params& p, cudaStream_t stream);
 
 }  // namespace logmel
 }  // namespace afs

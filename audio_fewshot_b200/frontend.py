@@ -4,7 +4,7 @@ The reference consumes pre-computed spectrogram folders and normalises them with
 [mean, std] pair of Auxiliary/*_Mean_Std.npy (libfewshot_core/test.py:398-399,
 audio_augmentations.py:36-53); it has no waveform code (SURVEY.md F2).  This module
 produces that `image` tensor [B, 1, 128, 157] directly from waveforms with ONE fused
-sm_100a kernel (csrc/logmel.cu).  Tables (periodic Hann, slaney mel filterbank) are
+sm_100a kernel (csrc/logmel_pair.cu; csrc/logmel.cu when augmenting).  Tables (periodic Hann, slaney mel filterbank) are
 computed here in float64 and rounded to fp32 once.
 """
 import math
@@ -60,9 +60,8 @@ class LogMelFrontEnd(nn.Module):
 
     def __init__(self, sample_rate=16000, n_fft=1024, hop_length=512, n_mels=128, f_min=0.0, f_max=None,
                  mean=0.0, std=1.0, mean_std_file=None, center=True, log_mult=10.0, log_eps=LOG_EPS, aug=None,
-                 seed=0, pcm_scale=1.0 / 32768.0, engine=None):
+                 seed=0, pcm_scale=1.0 / 32768.0):
         super().__init__()
-        self.engine = engine
         if mean_std_file is not None:
             mean, std = load_mean_std(mean_std_file)
         self.sample_rate, self.n_fft, self.hop_length, self.n_mels = sample_rate, n_fft, hop_length, n_mels
@@ -77,7 +76,7 @@ class LogMelFrontEnd(nn.Module):
     def plan(self):
         if self._plan is None:
             self._plan = ops.LogMelPlan(self._fb, self._window, self.hop_length, self.n_mels, self.center,
-                                        self.log_mult, self.log_eps, device=self.mean.device, engine=self.engine)
+                                        self.log_mult, self.log_eps, device=self.mean.device)
         return self._plan
 
     def forward(self, wav, first_clip_index=0, out=None):

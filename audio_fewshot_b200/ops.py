@@ -43,12 +43,15 @@ def _need_cuda(t, name, dtype=torch.float32):
 
 # --------------------------------------------------------------------------- front-end
 class LogMelPlan:
-    """Owns an afs_logmel_plan (device tables: window, twiddles, packed mel bands)."""
+    """Owns an afs_logmel_plan (device tables: window, twiddles, packed mel bands).  Plain launches run the pair
+    engine, augmented ones the radix-8 engine (include/afs_b200.h)."""
 
-    ENGINES = {"fft": 0, "pair": 2, "auto": 3}
+    @property
+    def engine(self):  # names that fixed rule; bench.py reads it to stamp logmel_engine
+        return "auto"
 
     def __init__(self, fb, window, hop, n_mels, center=True, log_mult=10.0, log_eps=2.220446049250313e-16,
-                 device=None, engine=None):
+                 device=None):
         if device is None:
             device = torch.cuda.current_device()
         device = torch.device("cuda", device) if isinstance(device, int) else torch.device(device)
@@ -67,17 +70,6 @@ class LogMelPlan:
         _lib.check(h.afs_logmel_plan_create(C.byref(self.cfg), fb.ctypes.data_as(C.c_void_p),
                                             window.ctypes.data_as(C.c_void_p), device.index,
                                             C.byref(self._handle)), "afs_logmel_plan_create")
-        self.engine = "auto"
-        if engine is not None:
-            self.set_engine(engine)
-
-    def set_engine(self, engine):
-        """"pair": two frames per warp as one 1024-point complex FFT; "fft": one frame per 64 threads, radix-8;
-        "auto" (default): "pair", "fft" for augmented launches.  Any other name raises ValueError."""
-        if engine not in self.ENGINES:
-            raise ValueError("unknown log-mel engine %r; expected one of %s" % (engine, sorted(self.ENGINES)))
-        _lib.check(_lib.lib().afs_logmel_plan_set_engine(self._handle, self.ENGINES[engine]), "afs_logmel_plan_set_engine")
-        self.engine = engine
 
     def num_frames(self, L):
         return int(_lib.lib().afs_logmel_num_frames(self._handle, int(L)))

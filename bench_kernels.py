@@ -61,21 +61,20 @@ def main():
     # ---- fused log-mel, shapes S5 and S1
     for tag, L, hop, B in (("S5 L=80000 hop=512", 80000, 512, 800), ("S5 L=80000 hop=512", 80000, 512, 3200),
                            ("S1 L=16000 hop=102", 16000, 102, 800)):
-        for engine, kname in (("pair", "logmel_pair_kernel<false> (warp-per-frame-pair engine, default)"),
-                              ("fft", "logmel_kernel<false> (radix-8 engine)")):
-            fr = LogMelFrontEnd(hop_length=hop, n_mels=128, mean=-15.0, std=26.0, engine=engine).to(dev).eval()
-            wav = torch.randn(B, L, device=dev) * 0.1
-            T = 1 + L // hop
-            out = torch.empty(B, 1, 128, T, device=dev)
-            ms, mn = timeit(lambda: fr(wav, out=out), flush=flush)
-            report("%s %s B=%d" % (kname, tag, B), "clip", B, 4 * L + 4 * 128 * T, ms, mn, note="T=%d" % T)
-            del wav, out
+        fr = LogMelFrontEnd(hop_length=hop, n_mels=128, mean=-15.0, std=26.0).to(dev).eval()
+        wav = torch.randn(B, L, device=dev) * 0.1
+        T = 1 + L // hop
+        out = torch.empty(B, 1, 128, T, device=dev)
+        ms, mn = timeit(lambda: fr(wav, out=out), flush=flush)
+        report("logmel_pair_kernel (warp-per-frame-pair engine, plain launches) %s B=%d" % (tag, B), "clip", B,
+               4 * L + 4 * 128 * T, ms, mn, note="T=%d" % T)
+        del wav, out
     fr = LogMelFrontEnd(hop_length=512, n_mels=128, mean=-15.0, std=26.0, seed=7,
                         aug={"gain_db": (-6.0, 6.0), "max_shift": 1600, "noise_std": (0.0, 0.02)}).to(dev).train()
     wav = torch.randn(800, 80000, device=dev) * 0.1
     out = torch.empty(800, 1, 128, 157, device=dev)
     ms, mn = timeit(lambda: fr(wav, out=out), flush=flush)
-    report("logmel_kernel<true> S5 + Philox gain/shift/noise", "clip", 800, 4 * 80000 + 4 * 128 * 157, ms, mn)
+    report("logmel_kernel (radix-8 engine, augmented launches) S5 + Philox gain/shift/noise", "clip", 800, 4 * 80000 + 4 * 128 * 157, ms, mn)
 
     # ---- conv1 stem
     img = torch.randn(800, 1, 128, 157, device=dev)
@@ -185,7 +184,7 @@ def extra():
     pcm = (torch.randn(800, 80000, device=dev) * 0.1 * 32768).round().clamp(-32768, 32767).to(torch.int16)
     out = torch.empty(800, 1, 128, 157, device=dev)
     ms, mn = timeit(lambda: fr(pcm, out=out), flush=flush)
-    report("logmel_kernel<false, int16> S5 (16-bit PCM input)", "clip", 800, 2 * 80000 + 4 * 128 * 157, ms, mn)
+    report("logmel_pair_kernel<int16> S5 (16-bit PCM input)", "clip", 800, 2 * 80000 + 4 * 128 * 157, ms, mn)
 
     img = torch.randn(800, 1, 128, 157, device=dev)
     for t in ("noise_suppression", "background_subtraction", "cutout"):

@@ -89,23 +89,14 @@ typedef struct afs_logmel_plan afs_logmel_plan; /* opaque; owns device tables */
 int afs_logmel_plan_create(const afs_logmel_cfg* cfg, const float* fb_host,
                            const float* window_host, int device, afs_logmel_plan** plan_out);
 int afs_logmel_plan_destroy(afs_logmel_plan* plan);
-/* Two engines compute the same features (each within the 1e-4 dB tolerance of the float64 spec):
- *   AFS_LOGMEL_ENGINE_FFT   one frame per 64 threads: 512-point complex radix-8 FFT in registers on the FMA pipe
- *                           (packed-f32x2 arithmetic), three shared-memory exchanges per frame, csrc/logmel.cu
- *   AFS_LOGMEL_ENGINE_PAIR  two frames per warp as ONE 1024-point complex FFT (32 x 32 in registers): one exchange per
- *                           frame pair, in-warp shuffle split, csrc/logmel_pair.cu -- the fastest for plain launches
- *   AFS_LOGMEL_ENGINE_AUTO  (default) PAIR, except FFT when waveform augmentation is requested (its Philox draws are
- *                           shared by sample pairs there)
- * The numbering is part of the ABI and has a gap at 1; any other value returns AFS_ERR_INVALID_ARG.          */
-#define AFS_LOGMEL_ENGINE_FFT 0
-#define AFS_LOGMEL_ENGINE_PAIR 2
-#define AFS_LOGMEL_ENGINE_AUTO 3
-int afs_logmel_plan_set_engine(afs_logmel_plan* plan, int32_t engine);
 /* number of output frames for clips of L samples */
 int afs_logmel_num_frames(const afs_logmel_plan* plan, int64_t L);
 
 /* wav [B, L] fp32; mean/std [n_mels] fp32 (per-bin; broadcast the scalar of
- * Auxiliary/<set>_Mean_Std.npy into it); aug nullable; out [B, 1, n_mels, T].  */
+ * Auxiliary/<set>_Mean_Std.npy into it); aug nullable; out [B, 1, n_mels, T].
+ * Both entry points run the pair engine (two frames per warp as one 1024-point FFT, csrc/logmel_pair.cu) when aug is
+ * null and the radix-8 engine (one frame per 64 threads, csrc/logmel.cu) otherwise, because the pair engine's lanes
+ * hold samples 32 apart and would evaluate each Philox block, shared by a sample pair, twice.  */
 int afs_logmel_fwd(const afs_logmel_plan* plan, const float* wav, int32_t B, int64_t L,
                    const float* mean, const float* std, const afs_aug_cfg* aug,
                    uint64_t seed, uint64_t first_clip_index, float* out, afs_stream_t stream);
