@@ -142,9 +142,12 @@ def build_model(config, device, arch=None, mode="train"):
 
 
 def frontend_from_config(config, device, **overrides):
-    """LogMelFrontEnd normalised with the config's `mean_std_file` (Auxiliary/*_Mean_Std.npy)."""
+    """LogMelFrontEnd normalised with the config's `mean_std_file` (Auxiliary/*_Mean_Std.npy), at the config's
+    `sample_rate`, `n_fft` and `hop_length` (defaults 16000 / 1024 / 512; e.g. 32000 / 2048 / 1024 or
+    8000 / 512 / 256 give the same 157 frames for 5 s clips at their own rate)."""
     from .frontend import LogMelFrontEnd
-    kw = dict(sample_rate=16000, n_fft=1024, hop_length=512, n_mels=128)
+    kw = dict(sample_rate=int(config.get("sample_rate", 16000)), n_fft=int(config.get("n_fft", 1024)),
+              hop_length=int(config.get("hop_length", 512)), n_mels=128)
     kw.update(overrides)
     path = config.get("mean_std_file")
     if path and os.path.exists(path):

@@ -1,5 +1,6 @@
 // Fused waveform -> normalised log-mel front-end for sm_100a: the plan, the C ABI entry points, and the radix-8
-// engine, which serves augmented launches (plain launches run the pair engine of logmel_pair.cu).
+// engine, which serves augmented launches at n_fft 1024 (plain launches at 1024 run the pair engine of
+// logmel_pair.cu; n_fft 512 and 2048 run logmel_nfft.cu).
 //
 // One launch does: Philox gain / time-shift / additive-noise
 // augmentation -> reflect padding -> framing -> window -> 1024-point real FFT
@@ -204,22 +205,24 @@ extern "C" int afs_logmel_plan_create(const afs_logmel_cfg* cfg, const float* fb
   if (cfg == nullptr || fb_host == nullptr || window_host == nullptr || plan_out == nullptr)
     return AFS_ERR_INVALID_ARG;
   if (cfg->hop < 1 || cfg->n_mels < 1) return AFS_ERR_INVALID_ARG;
-  if (cfg->n_fft != kNfft || cfg->n_mels > kMaxMels) return AFS_ERR_UNSUPPORTED;
+  const int n_fft = cfg->n_fft;
+  if ((n_fft != 512 && n_fft != kNfft && n_fft != 2048) || cfg->n_mels > kMaxMels) return AFS_ERR_UNSUPPORTED;
 
   std::vector<int> band;
   std::vector<float> weights;
-  pack_mel_ell(fb_host, cfg->n_mels, band, weights);
-  if (weights.size() > static_cast<size_t>(kMaxNnz)) return AFS_ERR_UNSUPPORTED;
+  pack_mel_ell(fb_host, cfg->n_mels, n_fft / 2 + 1, band, weights);
+  const int max_nnz = n_fft == kNfft ? kMaxNnz : logmel::nfft_max_nnz(n_fft);
+  if (weights.size() > static_cast<size_t>(max_nnz)) return AFS_ERR_UNSUPPORTED;
   if (weights.empty()) weights.push_back(0.f);
   std::vector<int> band64;
   std::vector<float> weights64;
-  pack_mel_ell(fb_host, cfg->n_mels, band64, weights64, logmel::kBanks64);
+  pack_mel_ell(fb_host, cfg->n_mels, n_fft / 2 + 1, band64, weights64, logmel::kBanks64);
   weights64.resize(weights.size(), 0.f);  // same rows per warp-pass, only the start shifts differ
 
-  std::vector<float2> tw(kNfft);
+  std::vector<float2> tw(n_fft);
   const double two_pi = 6.283185307179586476925286766559;
-  for (int k = 0; k < kNfft; ++k) {
-    const double a = two_pi * k / kNfft;
+  for (int k = 0; k < n_fft; ++k) {
+    const double a = two_pi * k / n_fft;
     tw[k] = make_float2(static_cast<float>(cos(a)), static_cast<float>(-sin(a)));
   }
 
@@ -234,12 +237,12 @@ extern "C" int afs_logmel_plan_create(const afs_logmel_cfg* cfg, const float* fb
   int prev = 0;
   cudaError_t e = cudaGetDevice(&prev);
   if (e == cudaSuccess) e = cudaSetDevice(device);
-  if (e == cudaSuccess) e = cudaMalloc(&plan->d_window, kNfft * sizeof(float));
-  if (e == cudaSuccess) e = cudaMalloc(&plan->d_tw1024, kNfft * sizeof(float2));
+  if (e == cudaSuccess) e = cudaMalloc(&plan->d_window, n_fft * sizeof(float));
+  if (e == cudaSuccess) e = cudaMalloc(&plan->d_tw1024, n_fft * sizeof(float2));
   if (e == cudaSuccess) e = cudaMalloc(&plan->d_band, band.size() * sizeof(int));
   if (e == cudaSuccess) e = cudaMalloc(&plan->d_weights, weights.size() * sizeof(float));
-  if (e == cudaSuccess) e = cudaMemcpy(plan->d_window, window_host, kNfft * sizeof(float), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemcpy(plan->d_tw1024, tw.data(), kNfft * sizeof(float2), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy(plan->d_window, window_host, n_fft * sizeof(float), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy(plan->d_tw1024, tw.data(), n_fft * sizeof(float2), cudaMemcpyHostToDevice);
   if (e == cudaSuccess) e = cudaMemcpy(plan->d_band, band.data(), band.size() * sizeof(int), cudaMemcpyHostToDevice);
   if (e == cudaSuccess) e = cudaMemcpy(plan->d_weights, weights.data(), weights.size() * sizeof(float), cudaMemcpyHostToDevice);
   if (e == cudaSuccess) e = cudaMalloc(&plan->d_band64, band64.size() * sizeof(int));
@@ -249,7 +252,7 @@ extern "C" int afs_logmel_plan_create(const afs_logmel_cfg* cfg, const float* fb
   const int smem = static_cast<int>(kSmemBytes);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(logmel_kernel<int16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e == cudaSuccess) e = logmel::pair_prepare();
+  if (e == cudaSuccess) e = n_fft == kNfft ? logmel::pair_prepare() : logmel::nfft_prepare(n_fft);
   cudaSetDevice(prev);
   if (e != cudaSuccess) {
     afs_logmel_plan_destroy(plan);
@@ -287,7 +290,7 @@ int logmel_launch(const afs_logmel_plan* plan, const S* wav, float pcm_scale, in
       B < 0 || L < 1)
     return AFS_ERR_INVALID_ARG;
   const afs_logmel_cfg& cfg = plan->cfg;
-  const int pad = cfg.center ? kNfft / 2 : 0;
+  const int pad = cfg.center ? cfg.n_fft / 2 : 0;
   if (cfg.center && L <= pad) return AFS_ERR_INVALID_ARG;  // reflect padding needs pad < L
   if (aug != nullptr && (aug->max_shift < 0 || aug->noise_std_lo < 0.f || aug->noise_std_hi < aug->noise_std_lo ||
                          aug->gain_db_hi < aug->gain_db_lo))
@@ -304,13 +307,16 @@ int logmel_launch(const afs_logmel_plan* plan, const S* wav, float pcm_scale, in
   const int64_t items = static_cast<int64_t>(B) * p.chunks;
   if (items > 0x7fffffffLL) return AFS_ERR_UNSUPPORTED;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (aug == nullptr) return logmel::pair_launch<S>(plan, p, stream);
+  if (aug == nullptr && cfg.n_fft == kNfft) return logmel::pair_launch<S>(plan, p, stream);
 
-  p.gain_lo = aug->gain_db_lo; p.gain_hi = aug->gain_db_hi;
-  p.noise_lo = aug->noise_std_lo; p.noise_hi = aug->noise_std_hi;
-  p.max_shift = aug->max_shift;
+  if (aug != nullptr) {  // a plain launch of the n_fft 512 / 2048 kernel keeps the zero ranges: gain 1, no shift, no noise
+    p.gain_lo = aug->gain_db_lo; p.gain_hi = aug->gain_db_hi;
+    p.noise_lo = aug->noise_std_lo; p.noise_hi = aug->noise_std_hi;
+    p.max_shift = aug->max_shift;
+  }
   p.seed_lo = static_cast<uint32_t>(seed); p.seed_hi = static_cast<uint32_t>(seed >> 32);
   p.first_clip = first_clip_index;
+  if (cfg.n_fft != kNfft) return logmel::nfft_launch<S>(plan, p, stream);
   // persistent: 2 resident CTAs per SM (128 registers x 256 threads, 100 KB of shared memory each) walk the items
   const unsigned grid = static_cast<unsigned>(items < 2 * kNumSMs ? items : 2 * kNumSMs);
   logmel_kernel<S><<<grid, kThreads, kSmemBytes, stream>>>(p);

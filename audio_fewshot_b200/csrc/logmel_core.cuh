@@ -89,16 +89,16 @@ AFS_HD float norm_db(float e, float eps, float scale, float shift) {
   return fast_log2(e + eps) * scale + shift;
 }
 
-// Host-side packing of a dense [kBins, n_mels] filterbank into per-filter spans:
+// Host-side packing of a dense [bins, n_mels] filterbank (bins = n_fft/2 + 1) into per-filter spans:
 // band[m] = first non-zero bin, band[kMaxMels+m] = span length, band[2*kMaxMels+m] = offset
 // into `weights`.  Returns the number of packed weights.
 template <typename IntVec, typename FloatVec>
-inline int pack_mel_bands(const float* fb, int n_mels, IntVec& band, FloatVec& weights) {
+inline int pack_mel_bands(const float* fb, int n_mels, int bins, IntVec& band, FloatVec& weights) {
   band.assign(3 * kMaxMels, 0);
   weights.clear();
   for (int m = 0; m < n_mels; ++m) {
     int lo = -1, hi = -1;
-    for (int k = 0; k < kBins; ++k) {
+    for (int k = 0; k < bins; ++k) {
       if (fb[static_cast<size_t>(k) * n_mels + m] != 0.f) {
         if (lo < 0) lo = k;
         hi = k;
@@ -111,6 +111,10 @@ inline int pack_mel_bands(const float* fb, int n_mels, IntVec& band, FloatVec& w
     for (int i = 0; i < len; ++i) weights.push_back(fb[static_cast<size_t>(lo + i) * n_mels + m]);
   }
   return static_cast<int>(weights.size());
+}
+template <typename IntVec, typename FloatVec>
+inline int pack_mel_bands(const float* fb, int n_mels, IntVec& band, FloatVec& weights) {
+  return pack_mel_bands(fb, n_mels, kBins, band, weights);
 }
 
 // Shared-memory wavefronts of one warp-pass of the mel projection for one frame: in iteration i lane l reads power
@@ -157,10 +161,11 @@ inline int mel_read_wavefronts(const int (&start)[32], const int (&n)[32], MelBa
 //   band[2*kMaxMels+m] = index of the filter's table entry 0; consecutive entries are kEllStride apart.
 constexpr int kEllStride = 32;
 template <typename IntVec, typename FloatVec>
-inline int pack_mel_ell(const float* fb, int n_mels, IntVec& band, FloatVec& weights, MelBankModel model = kBanks32) {
+inline int pack_mel_ell(const float* fb, int n_mels, int bins, IntVec& band, FloatVec& weights,
+                        MelBankModel model = kBanks32) {
   IntVec b0;
   FloatVec w0;
-  pack_mel_bands(fb, n_mels, b0, w0);
+  pack_mel_bands(fb, n_mels, bins, b0, w0);
   band.assign(3 * kMaxMels, 0);
   weights.clear();
   for (int pass = 0; pass < 2; ++pass) {
@@ -213,6 +218,10 @@ inline int pack_mel_ell(const float* fb, int n_mels, IntVec& band, FloatVec& wei
     }
   }
   return static_cast<int>(weights.size());
+}
+template <typename IntVec, typename FloatVec>
+inline int pack_mel_ell(const float* fb, int n_mels, IntVec& band, FloatVec& weights, MelBankModel model = kBanks32) {
+  return pack_mel_ell(fb, n_mels, kBins, band, weights, model);
 }
 
 }  // namespace logmel

@@ -12,8 +12,8 @@ struct afs_logmel_plan {
   afs_logmel_cfg cfg;
   int device;
   int nnz;
-  float* d_window;   // [1024]
-  float2* d_tw1024;  // [1024]
+  float* d_window;   // [n_fft]
+  float2* d_tw1024;  // [n_fft]: (cos, -sin)(2 pi k / n_fft)
   int* d_band;       // [3][128]: lo, len, off
   float* d_weights;  // [nnz]
   int* d_band64;     // the same table with start shifts chosen for 64-bit power reads (pair engine)
@@ -23,7 +23,7 @@ struct afs_logmel_plan {
 namespace afs {
 namespace logmel {
 
-struct Params {
+struct Params {  // tw1024 carries the plan's n_fft-point table; the name is the 1024-point engines'.
   const void* wav;     // [B, L] fp32, or int16 PCM when launched with T = int16_t
   float pcm_scale;     // int16 PCM only: sample = (float)pcm * pcm_scale (1/32768 for full-scale [-1, 1))
   float* out;
@@ -127,6 +127,12 @@ inline int num_frames(const afs_logmel_cfg& cfg, int64_t L) {
 cudaError_t pair_prepare();
 template <typename S>
 int pair_launch(const afs_logmel_plan* plan, const Params& p, cudaStream_t stream);
+
+// logmel_nfft.cu: n_fft 512 and 2048, plain and augmented launches
+cudaError_t nfft_prepare(int n_fft);
+int nfft_max_nnz(int n_fft);  // floats of the ELL weight table the kernel stages
+template <typename S>
+int nfft_launch(const afs_logmel_plan* plan, const Params& p, cudaStream_t stream);
 
 }  // namespace logmel
 }  // namespace afs

@@ -4,7 +4,7 @@ The reference consumes pre-computed spectrogram folders and normalises them with
 [mean, std] pair of Auxiliary/*_Mean_Std.npy (libfewshot_core/test.py:398-399,
 audio_augmentations.py:36-53); it has no waveform code (SURVEY.md F2).  This module
 produces that `image` tensor [B, 1, 128, 157] directly from waveforms with ONE fused
-sm_100a kernel (csrc/logmel_pair.cu; csrc/logmel.cu when augmenting).  Tables (periodic Hann, slaney mel filterbank) are
+sm_100a kernel (csrc/logmel_pair.cu; csrc/logmel.cu when augmenting; csrc/logmel_nfft.cu at n_fft 512 and 2048).  Tables (periodic Hann, slaney mel filterbank) are
 computed here in float64 and rounded to fp32 once.
 """
 import math
@@ -56,7 +56,9 @@ def load_mean_std(path):
 
 class LogMelFrontEnd(nn.Module):
     """wav [B, L] (CUDA fp32, or int16 PCM read as pcm * pcm_scale) -> [B, 1, n_mels, T].
-    mean/std: scalars or per-bin [n_mels]."""
+    mean/std: scalars or per-bin [n_mels].  n_fft 512, 1024 or 2048 (other sizes raise AfsError on the first call):
+    e.g. 8 kHz audio with n_fft 512 / hop 256, 32 kHz with 2048 / 1024 -- 5 s clips give the [1, 128, 157] image of
+    16 kHz / 1024 / 512 at the audio's own rate."""
 
     def __init__(self, sample_rate=16000, n_fft=1024, hop_length=512, n_mels=128, f_min=0.0, f_max=None,
                  mean=0.0, std=1.0, mean_std_file=None, center=True, log_mult=10.0, log_eps=LOG_EPS, aug=None,

@@ -43,8 +43,10 @@ def _need_cuda(t, name, dtype=torch.float32):
 
 # --------------------------------------------------------------------------- front-end
 class LogMelPlan:
-    """Owns an afs_logmel_plan (device tables: window, twiddles, packed mel bands).  Plain launches run the pair
-    engine, augmented ones the radix-8 engine (include/afs_b200.h)."""
+    """Owns an afs_logmel_plan (device tables: window, twiddles, packed mel bands).  n_fft is the window's length:
+    512, 1024 or 2048 (AfsError otherwise); fb is [n_fft/2+1, n_mels], n_mels <= 128.  At n_fft 1024 plain launches
+    run the pair engine and augmented ones the radix-8 engine; at 512 and 2048 every launch runs logmel_nfft_kernel
+    (include/afs_b200.h)."""
 
     @property
     def engine(self):  # names that fixed rule; bench.py reads it to stamp logmel_engine

@@ -217,6 +217,55 @@ def extra():
            4 * 128 * 157 * 3 + 2 * 4 * 64 * 42 * 52, ms_fb, mn_fb, flops_per_unit=3 * 2 * 64 * 42 * 52 * 81)
 
 
+def logmel_nfft():
+    """The front-end at n_fft 512 (8 kHz, hop 256) and 2048 (32 kHz, hop 1024): 5 s clips -> [3200, 1, 128, 157], plain,
+    augmented and int16 launches of logmel_nfft_kernel, the torch.stft -> |.|^2 -> matmul -> log10 sequence at the same
+    shapes, and time per frame against the n_fft 1024 radix-8 engine (logmel_kernel, zero-range augmented launch) at
+    16 kHz / hop 512, which transforms the same 3200 x 157 frames."""
+    from oracle import frontend as ofe
+    dev = torch.device("cuda", 0)
+    flush = torch.empty(160 * 2 ** 20 // 4, dtype=torch.float32, device=dev)
+    B, T = 3200, 157
+    zero = {"gain_db": (0.0, 0.0), "max_shift": 0, "noise_std": (0.0, 0.0)}
+    real = {"gain_db": (-6.0, 6.0), "max_shift": 1600, "noise_std": (0.0, 0.02)}
+    fr = LogMelFrontEnd(hop_length=512, n_mels=128, mean=-15.0, std=26.0, aug=zero).to(dev).train()
+    wav = torch.randn(B, 80000, device=dev) * 0.1
+    out = torch.empty(B, 1, 128, T, device=dev)
+    ms_1024, mn = timeit(lambda: fr(wav, out=out), flush=flush)
+    report("logmel_kernel (n_fft 1024 radix-8 engine, zero-range augmented launch) 16 kHz hop 512 B=%d" % B, "clip", B,
+           4 * 80000 + 4 * 128 * T, ms_1024, mn, note="reference for the per-frame ratios below")
+    del wav
+    for tag, sr, n_fft, hop, L in (("8 kHz n_fft 512 hop 256", 8000, 512, 256, 40000),
+                                   ("32 kHz n_fft 2048 hop 1024", 32000, 2048, 1024, 160000)):
+        wav = torch.randn(B, L, device=dev) * 0.1
+        pcm = (wav * 32768).round().clamp(-32768, 32767).to(torch.int16)
+        nb = 4 * L + 4 * 128 * T
+        for launch, aug, x, nbytes in (("plain", None, wav, nb), ("augmented (Philox gain/shift/noise)", real, wav, nb),
+                                       ("plain, int16 PCM input", None, pcm, nb - 2 * L)):
+            f = LogMelFrontEnd(sr, n_fft=n_fft, hop_length=hop, n_mels=128, mean=-15.0, std=26.0, seed=7,
+                               aug=aug).to(dev)
+            f = f.train() if aug else f.eval()
+            ms, mn = timeit(lambda: f(x, out=out), flush=flush)
+            report("logmel_nfft_kernel<%d> %s, %s B=%d" % (n_fft, tag, launch, B), "clip", B, nbytes, ms, mn,
+                   note="T=%d; time per frame / n_fft 1024 radix-8 engine = %.2f" % (T, ms / ms_1024))
+        win = torch.from_numpy(ofe.hann_periodic(n_fft)).to(dev)
+        fb = torch.from_numpy(ofe.mel_filterbank(n_fft // 2 + 1, 0.0, sr / 2.0, 128, sr)).to(dev)
+
+        def torch_path():
+            spec = torch.stft(wav, n_fft, hop, n_fft, win, center=True, pad_mode="reflect", return_complex=True)
+            mel = torch.matmul((spec.real ** 2 + spec.imag ** 2).transpose(1, 2), fb).transpose(1, 2)
+            return ((10 * torch.log10(mel + ofe.LOG_EPS) + 15.0) / 26.0).unsqueeze(1)
+
+        ms, mn = timeit(torch_path, iters=5, flush=flush)
+        report("torch.stft -> |.|^2 -> matmul -> log10 %s B=%d" % (tag, B), "clip", B, 4 * L + 4 * 128 * T, ms, mn,
+               note="PyTorch op sequence at the same shape (cuFFT + GEMM; the spectrum goes through HBM)")
+        del wav, pcm
+
+
 if __name__ == "__main__":
-    main()
-    extra()
+    if "--logmel-nfft" in sys.argv:
+        logmel_nfft()
+    else:
+        main()
+        extra()
+        logmel_nfft()

@@ -34,7 +34,7 @@ typedef void* afs_stream_t; /* cudaStream_t */
 typedef enum afs_status {
   AFS_OK = 0,
   AFS_ERR_INVALID_ARG = -1,  /* null pointer, negative size, unsupported shape */
-  AFS_ERR_UNSUPPORTED = -2,  /* valid but not built (e.g. n_fft != 1024)       */
+  AFS_ERR_UNSUPPORTED = -2,  /* valid but not built (e.g. n_fft not 512/1024/2048) */
   AFS_ERR_CUDA = -3,         /* a CUDA runtime call failed; see afs_last_cuda_error */
   AFS_ERR_WORKSPACE = -4     /* workspace too small                              */
 } afs_status;
@@ -61,7 +61,7 @@ uint64_t afs_launch_count(void);
  * No spectrum is ever written to HBM.
  * ---------------------------------------------------------------------- */
 typedef struct afs_logmel_cfg {
-  int32_t n_fft;    /* 1024 (the only size built)                       */
+  int32_t n_fft;    /* 512, 1024 or 2048 (8 kHz / 16 kHz / 32-48 kHz)   */
   int32_t hop;      /* >= 1                                             */
   int32_t n_mels;   /* 1..128                                           */
   int32_t center;   /* 1: reflect padding of n_fft/2 on both sides      */
@@ -84,8 +84,9 @@ typedef struct afs_logmel_plan afs_logmel_plan; /* opaque; owns device tables */
  * melscale_fbanks layout); window_host: [n_fft].  Both HOST pointers; the
  * plan packs each filter's contiguous non-zero band and uploads it together
  * with the window and the FFT twiddles.  device: CUDA device ordinal.
- * AFS_ERR_UNSUPPORTED when the packed table exceeds the kernel's 16 KB budget (very wide filters: fewer than
- * about 30 slaney mels at n_fft 1024). */
+ * AFS_ERR_UNSUPPORTED for any other n_fft, n_mels > 128, or when the packed table exceeds the kernel's budget
+ * (16 KB at n_fft 512 and 1024, 32 KB at 2048; very wide filters: fewer than about 30 slaney mels at 1024, fewer
+ * than about 48 at 32-48 kHz and 2048). */
 int afs_logmel_plan_create(const afs_logmel_cfg* cfg, const float* fb_host,
                            const float* window_host, int device, afs_logmel_plan** plan_out);
 int afs_logmel_plan_destroy(afs_logmel_plan* plan);
@@ -94,9 +95,11 @@ int afs_logmel_num_frames(const afs_logmel_plan* plan, int64_t L);
 
 /* wav [B, L] fp32; mean/std [n_mels] fp32 (per-bin; broadcast the scalar of
  * Auxiliary/<set>_Mean_Std.npy into it); aug nullable; out [B, 1, n_mels, T].
- * Both entry points run the pair engine (two frames per warp as one 1024-point FFT, csrc/logmel_pair.cu) when aug is
- * null and the radix-8 engine (one frame per 64 threads, csrc/logmel.cu) otherwise, because the pair engine's lanes
- * hold samples 32 apart and would evaluate each Philox block, shared by a sample pair, twice.  */
+ * At n_fft 1024 both entry points run the pair engine (two frames per warp as one 1024-point FFT,
+ * csrc/logmel_pair.cu) when aug is null and the radix-8 engine (one frame per 64 threads, csrc/logmel.cu) otherwise,
+ * because the pair engine's lanes hold samples 32 apart and would evaluate each Philox block, shared by a sample pair,
+ * twice.  At n_fft 512 and 2048 every launch runs csrc/logmel_nfft.cu (one frame per 64 threads, radix-4 / radix-16
+ * register pass + two radix-8 cross-thread passes).  */
 int afs_logmel_fwd(const afs_logmel_plan* plan, const float* wav, int32_t B, int64_t L,
                    const float* mean, const float* std, const afs_aug_cfg* aug,
                    uint64_t seed, uint64_t first_clip_index, float* out, afs_stream_t stream);
