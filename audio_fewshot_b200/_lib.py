@@ -129,6 +129,11 @@ SIGNATURES = {
     "afs_bdc_set_tensor_core": (C.c_int, [C.c_int32]),
     "afs_bdc_fwd": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32,
                               C.c_void_p, C.c_void_p]),
+    "afs_bdc_wide_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32]),
+    "afs_bdc_wide_fwd": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32,
+                                   C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "afs_bdc_wide_bwd": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p,
+                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "afs_spec_augment": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_float,
                                    C.POINTER(SpecAugCfg), C.c_void_p, C.c_void_p, C.c_void_p]),
     "afs_vote_acc": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32,

@@ -571,6 +571,16 @@ def dn4_scores(feat, cls_row, E, W, S, n_k, want_topk=False, want_pred=False, pr
     return score, topk, pred
 
 
+def _bdc_wide_ws(B, Cc, backward, device):
+    """Workspace of the 64-channel-block kernels (csrc/bdc_wide.cu) for C = 128, 192, ..., 640, else None: every other
+    channel count stays with afs_bdc_fwd / afs_bdc_bwd."""
+    h = _lib.lib()
+    if h.afs_bdc_wide_workspace_bytes(1, Cc, 0) == 0:
+        return None
+    return torch.empty((int(h.afs_bdc_wide_workspace_bytes(B, Cc, 1 if backward else 0)),), dtype=torch.uint8,
+                       device=device)
+
+
 def _bdc_call(x, log_temp, triu):
     _need_cuda(x, "x")
     _need_cuda(log_temp, "log_temp")
@@ -579,6 +589,11 @@ def _bdc_call(x, log_temp, triu):
     M = int(np.prod(x.shape[2:]))
     out_dim = Cc * (Cc + 1) // 2 if triu else Cc * Cc
     out = torch.empty((B, out_dim), dtype=torch.float32, device=x.device)
+    ws = _bdc_wide_ws(B, Cc, False, x.device)
+    if ws is not None:
+        _lib.check(_lib.lib().afs_bdc_wide_fwd(_ptr(x), B, Cc, M, _ptr(log_temp.contiguous()), 1 if triu else 0,
+                                               _ptr(out), _ptr(ws), ws.numel(), _stream()), "afs_bdc_wide_fwd")
+        return x, out
     _lib.check(_lib.lib().afs_bdc_fwd(_ptr(x), B, Cc, M, _ptr(log_temp.contiguous()), 1 if triu else 0, _ptr(out),
                                       _stream()), "afs_bdc_fwd")
     return x, out
@@ -601,6 +616,12 @@ class _BdcFn(torch.autograd.Function):
         grad_out = grad_out.contiguous().float()
         grad_x = torch.empty_like(x)
         grad_t = torch.empty((B,), dtype=torch.float32, device=x.device)
+        ws = _bdc_wide_ws(B, Cc, True, x.device)
+        if ws is not None:
+            _lib.check(_lib.lib().afs_bdc_wide_bwd(_ptr(x), B, Cc, M, _ptr(log_temp), 1 if ctx.triu else 0,
+                                                   _ptr(grad_out), _ptr(grad_x), _ptr(grad_t), _ptr(ws), ws.numel(),
+                                                   _stream()), "afs_bdc_wide_bwd")
+            return grad_x, grad_t.sum().reshape(ctx.t_shape), None
         _lib.check(_lib.lib().afs_bdc_bwd(_ptr(x), B, Cc, M, _ptr(log_temp), 1 if ctx.triu else 0, _ptr(grad_out),
                                           _ptr(grad_x), _ptr(grad_t), _stream()), "afs_bdc_bwd")
         return grad_x, grad_t.sum().reshape(ctx.t_shape), None
@@ -616,7 +637,8 @@ def bdc_pool(x, log_temp, triu=True):
 
 def bdc_set_tensor_core(enable):
     """Process-wide switch of afs_bdc_fwd: True (default) runs the Gram on tcgen05 where the shape allows
-    (C == 64, M % 4 == 0), False always the fp32 FMA kernel."""
+    (C == 64, M % 4 == 0), False always the fp32 FMA kernel.  C = 128, 192, ..., 640 always run the fp32 FMA kernels
+    of csrc/bdc_wide.cu, with the same bits either way."""
     _lib.check(_lib.lib().afs_bdc_set_tensor_core(1 if enable else 0), "afs_bdc_set_tensor_core")
 
 

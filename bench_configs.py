@@ -8,6 +8,8 @@ resident on the device) go through `model(batch_list)` exactly as test.py:380 / 
     C2  ProtoNet / resnet12  5w1s15q   eval   set_forward            (D = 12 800)
     C3  DN4 / Conv64F maps   5w5s15q   eval   set_forward, n_k = 3   (fp32 parity head and tcgen05 TF32 head)
     C4  DeepBDC / resnet12Bdc reduce_dim 64, 5w5s10q  eval  set_forward
+    C4w DeepBDC / resnet12Bdc at its default reduce_dim (640), 5w5s10q, eval, set_forward, with the BDC kernels' share
+        of the step's device time from torch.profiler (opt-in: --only C4w)
     C5  MAML / Conv64F       5w5s10q   train  set_forward_loss + backward, episode_size 2, 5 inner steps
 
 One JSON line per config on stdout; CUDA events, >= 3 warm-up steps, inputs rotate over two batches that together
@@ -37,6 +39,38 @@ def timeit(step, iters, warmup):
     t1.record()
     torch.cuda.synchronize()
     return t0.elapsed_time(t1) / iters
+
+
+def card():
+    """Name and power limit of the GPU the numbers were measured on."""
+    import subprocess
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
+                       capture_output=True, text=True).stdout.strip()
+    return "card: %s" % (q or torch.cuda.get_device_name(0))
+
+
+def bdc_share(model, E, W, S, Q, steps=5):
+    """Share of the step's kernel time spent in the bdc* kernels, from torch.profiler over `steps` warm steps (a run
+    of its own: the timed steps run without the profiler)."""
+    from torch.profiler import ProfilerActivity, profile
+    dev = torch.device("cuda", 0)
+    n = E * W * (S + Q)
+    x = images(n, dev, 400)
+    repeats = torch.ones(E * W * Q, dtype=torch.long)
+    model.eval()
+    with torch.no_grad():
+        for _ in range(2):
+            model([x, None, repeats, E * W * S])
+        torch.cuda.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            for _ in range(steps):
+                model([x, None, repeats, E * W * S])
+            torch.cuda.synchronize()
+    kernels = [e for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA]
+    total = sum(e.device_time_total for e in kernels)
+    bdc = sum(e.device_time_total for e in kernels if "bdc" in e.name)
+    return "BDC kernels %.3f ms of %.3f ms kernel time per step (%.1f %%)" % (
+        bdc / 1e3 / steps, total / 1e3 / steps, 100.0 * bdc / max(total, 1e-9))
 
 
 def main():
@@ -147,6 +181,12 @@ def main():
         emb = arch.resnet12Bdc(reduce_dim=64, num_channels=1)
         m = arch.DeepBDC(shot_num=5, query_num=10, test_shot=5, test_query=10, emb_func=emb, device=dev, **common).to(dev)
         run_eval("C4", "DeepBDC/resnet12Bdc(dr=64) 5w5s10q set_forward", m, 4, 5, 5, 10, "300 images per step")
+
+    if only is not None and "C4w" in only:
+        emb = arch.resnet12Bdc(num_channels=1)
+        m = arch.DeepBDC(shot_num=5, query_num=10, test_shot=5, test_query=10, emb_func=emb, device=dev, **common).to(dev)
+        run_eval("C4w", "DeepBDC/resnet12Bdc(default reduce_dim = 640) 5w5s10q set_forward", m, 4, 5, 5, 10,
+                 "300 images per step; " + bdc_share(m, 4, 5, 5, 10) + "; " + card())
 
     if only is None or "C5" in only:
         emb = arch.Conv64F(is_flatten=True, num_channels=1)

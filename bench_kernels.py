@@ -262,10 +262,66 @@ def logmel_nfft():
         del wav, pcm
 
 
+def _bdc_reference_fp32(x, t):
+    """The reference's op sequence (bdc_pool.py:69-93): BDCovpool's 7 bmm, 3 of them against an all-ones matrix, then
+    Triuvec's gather."""
+    B, C = x.shape[:2]
+    x = x.reshape(B, C, -1)
+    I = torch.eye(C, C, device=x.device).view(1, C, C).repeat(B, 1, 1)
+    I_M = torch.ones(B, C, C, device=x.device)
+    x_pow2 = x.bmm(x.transpose(1, 2))
+    dcov = I_M.bmm(x_pow2 * I) + (x_pow2 * I).bmm(I_M) - 2 * x_pow2
+    dcov = torch.sqrt(torch.exp(t) * torch.clamp(dcov, min=0.0) + 1e-5)
+    dcov = dcov - 1.0 / C * dcov.bmm(I_M) - 1.0 / C * I_M.bmm(dcov) + 1.0 / (C * C) * I_M.bmm(dcov).bmm(I_M)
+    index = torch.ones(C, C, device=x.device).triu().reshape(C * C).nonzero(as_tuple=False)
+    return dcov.reshape(B, C * C)[:, index].squeeze(-1)
+
+
+def bdc_wide():
+    """BDC at C = 128, 256, 640 on the 16 x 19 map (M = 304, resnet12Bdc's trunk output), B = 300 (one C4 step) and
+    2400 (input and output larger than L2): the 64-channel-block kernels of csrc/bdc_wide.cu, forward and forward +
+    backward, against the reference's fp32 op sequence at the same shapes with TF32 off.  Useful flops: the Gram with
+    its symmetry used, M C (C + 1) per clip, and for the backward also dX = S X, 2 C^2 M.  Bytes: x once, the
+    triangle once (forward); the backward adds grad_out, x and grad_x."""
+    dev = torch.device("cuda", 0)
+    flush = torch.empty(160 * 2 ** 20 // 4, dtype=torch.float32, device=dev)
+    torch.backends.cuda.matmul.allow_tf32 = False
+    t = torch.full((1, 1), float(np.log(1 / 200.0)), device=dev)
+    M = 304
+    for C in (128, 256, 640):
+        tri = C * (C + 1) // 2
+        fwd_bytes, fwd_flops = 4 * C * M + 4 * tri, M * C * (C + 1)
+        for B in (300, 2400):
+            x = torch.relu(torch.randn(B, C, 16, 19, device=dev))
+            ms, mn = timeit(lambda: ops.bdc_pool(x, t), flush=flush)
+            report("bdc_wide forward (norms + gram + center, fp32 FMA) C=%d M=%d B=%d" % (C, M, B), "clip", B, fwd_bytes,
+                   ms, mn, flops_per_unit=fwd_flops)
+            ms_ref, mn_ref = timeit(lambda: _bdc_reference_fp32(x, t), iters=5, flush=flush)
+            report("reference fp32 op sequence (7 bmm + Triuvec, TF32 off) C=%d M=%d B=%d" % (C, M, B), "clip", B,
+                   fwd_bytes, ms_ref, mn_ref, flops_per_unit=fwd_flops,
+                   note="same useful flops and bytes as the kernel row; bdc_wide forward is %.1fx faster" % (ms_ref / ms))
+            xg = x.clone().requires_grad_(True)
+            tg = t.clone().requires_grad_(True)
+            g = torch.randn(B, tri, device=dev)
+
+            def fwd_bwd():
+                ops.bdc_pool(xg, tg).backward(g)
+
+            ms, mn = timeit(fwd_bwd, flush=flush)
+            report("bdc_wide forward + backward (norms, gram, center; norms, dbstats, bwd_tile, dx) C=%d M=%d B=%d"
+                   % (C, M, B), "clip", B, fwd_bytes + 8 * C * M + 4 * tri, ms, mn,
+                   flops_per_unit=2 * fwd_flops + 2 * C * C * M)
+            del x, xg, g
+            torch.cuda.empty_cache()
+
+
 if __name__ == "__main__":
     if "--logmel-nfft" in sys.argv:
         logmel_nfft()
+    elif "--bdc-wide" in sys.argv:
+        bdc_wide()
     else:
         main()
         extra()
         logmel_nfft()
+        bdc_wide()

@@ -327,10 +327,12 @@ int afs_dn4_bwd(const float* feat, const int32_t* cls_row, int32_t N, int32_t E,
  * scale, sqrt, double centring, row-major upper triangle.  Replaces
  * BDCovpool + Triuvec (libfewshot_core/model/backbone/utils/bdc_pool.py:69-93).
  * x [B, C, M]; log_temp: device pointer to the scalar `temperature`;
- * out [B, C*(C+1)/2] if triu else [B, C*C].  C <= 64 built.  For C == 64 and
- * M % 4 == 0 (16-byte aligned x) the Gram runs on the tcgen05 tensor cores with 3 x TF32
- * operand splitting (csrc/bdc_tc.cu, within the same 1e-4 tolerance); other shapes, or
- * after afs_bdc_set_tensor_core(0), the fp32 FMA kernel of csrc/bdc.cu.           */
+ * out [B, C*(C+1)/2] if triu else [B, C*C].  afs_bdc_fwd / afs_bdc_bwd take C <= 64
+ * (AFS_ERR_UNSUPPORTED above); C = 128, 192, ..., 640 go to afs_bdc_wide_fwd / _bwd below.
+ * For C == 64 and M % 4 == 0 (16-byte aligned x) the Gram runs on the tcgen05 tensor cores
+ * with 3 x TF32 operand splitting (csrc/bdc_tc.cu, within the same 1e-4 tolerance); other
+ * shapes, or after afs_bdc_set_tensor_core(0), the fp32 FMA kernel of csrc/bdc.cu.  The
+ * switch has no effect on the wide entries.                                        */
 int afs_bdc_set_tensor_core(int32_t enable);
 int afs_bdc_fwd(const float* x, int32_t B, int32_t C, int32_t M, const float* log_temp,
                 int32_t triu, float* out, afs_stream_t stream);
@@ -340,6 +342,21 @@ int afs_bdc_fwd(const float* x, int32_t B, int32_t C, int32_t M, const float* lo
  * contributions to d loss / d temperature (the caller sums them).                           */
 int afs_bdc_bwd(const float* x, int32_t B, int32_t C, int32_t M, const float* log_temp, int32_t triu,
                 const float* grad_out, float* grad_x, float* grad_log_temp, afs_stream_t stream);
+
+/* (2c-wide) The same forward and backward for C = 128, 192, ..., 640 (whole 64-channel blocks; every other C returns
+ * AFS_ERR_UNSUPPORTED), any M >= 1, any B >= 0 (B == 0 is a no-op), both layouts; csrc/bdc_wide.cu.  fp32 on the FMA
+ * pipe, one CTA per clip and 64-channel block pair I <= J, no tensor cores whatever afs_bdc_set_tensor_core says.  A
+ * clip's output has the same bits whatever the batch size and its position in the batch; the full output is exactly
+ * symmetric.  ws: afs_bdc_wide_workspace_bytes(B, C, backward) bytes, 16-byte aligned (AFS_ERR_WORKSPACE if smaller
+ * or misaligned); the size is 0 for an unsupported C.  Forward: norms and per-tile row sums, 4 C (k + 1) bytes per
+ * clip (k = C / 64).  Backward: also dB's row and column sums and the k (k + 1) / 2 tiles of dD + dD^T, about
+ * 8 C^2 bytes per clip.                                                                                          */
+size_t afs_bdc_wide_workspace_bytes(int32_t B, int32_t C, int32_t backward);
+int afs_bdc_wide_fwd(const float* x, int32_t B, int32_t C, int32_t M, const float* log_temp, int32_t triu,
+                     float* out, void* ws, size_t ws_bytes, afs_stream_t stream);
+int afs_bdc_wide_bwd(const float* x, int32_t B, int32_t C, int32_t M, const float* log_temp, int32_t triu,
+                     const float* grad_out, float* grad_x, float* grad_log_temp, void* ws, size_t ws_bytes,
+                     afs_stream_t stream);
 
 /* (3) Window argmax -> per-query majority vote -> accuracy, all on device.
  * Replaces majority_vote + vote_catagorical_acc
